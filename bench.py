@@ -7,12 +7,24 @@ steps per probe, trace(exp(A)) by stochastic Lanczos quadrature.  One "step" = o
 (512 x 30 = 15 360 Krylov matvecs per GPU).  A is replicated, probes are sharded across ranks, one
 NCCL all-reduce of the partial trace per step (weak scaling: per-GPU work is fixed).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Metric: Krylov matvecs/sec (an n x k SpMM counts k).  `value` = device-resident probes;
 `e2e` = through the public host-buffer call kr_slq_trace (pinned host probes -> device, result back).
 `--impl reference` times the reference's CPU algorithm (the NumPy/SciPy oracle: the reference is
 MATLAB-only and cannot run here) on the host cores with the same metric.
+
+`--steps K` is the number of timed steps of every C3 arm (device probes, host probes, int8 sign probes, strong
+scaling); the C5, C4 and C2 arms time fixed calls.  At least 3 untimed steps precede the C3 timing whatever
+`--warmup` says with `--impl ours` (the first steps load modules and size the memory pool); the JSON line reports
+the number run.
+
+`--dump-outputs DIR` writes, after the run, what the timed calls returned to their caller as DIR/<name>.npy
+(float64): c3_trace (the trace of the last timed step), c5_edge_scores, c2_entries and c4_expmv_sample (4096
+seeded rows of the n x 64 result), each for the arms that ran.  All inputs are seeded, so the same arguments give
+the same inputs and two builds can be compared output for output.  The inputs that the device itself derives are
+written next to them, so that a difference there shows up as an input change: c5_candidates (the 1-based node
+pairs picked by the device centrality), c4_tscale (from the device norm estimate) and c2_tol (likewise).
 """
 import argparse
 import json
@@ -218,7 +230,13 @@ def peak_gbs():
         return 6650.0
 
 
-def bench_c2(kr, ctx):
+def dump_outputs(outdir, outputs):
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(outdir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
+def bench_c2(kr, ctx, outputs):
     """Config C2 (datasets_paper/Transport, gradient over ALL edges): gr = -2 cosh(A + Delta(X))_Omega on the largest road
     network of the reference's data (Vermont after the scripts' preprocessing, committed fixture), through
     function_multiple_entries - one single-vector Krylov space per distinct row index, each run whole in one CTA on the
@@ -253,6 +271,8 @@ def bench_c2(kr, ctx):
             ctx.sync()
             times.append(time.perf_counter() - t0)
         c1 = ctx.counters()
+    outputs["c2_entries"] = v
+    outputs["c2_tol"] = np.array([tol])
     t = min(times)
     return {"metric": "gradient_entries_per_sec", "value": Om.shape[0] / t, "unit": "entry/s",
             "workload": "C2: transport_Vermont (n=%d, %d edges), gradient of trace sinh(A+X) over ALL edges = %d entries of "
@@ -267,7 +287,7 @@ def bench_c2(kr, ctx):
             "note": "round-2 dense batch (all spaces advanced by n x R SpMMs): 11.5-11.9 s for the same call, see DESIGN.md 6"}
 
 
-def bench_c4(kr, ctx):
+def bench_c4(kr, ctx, outputs):
     """expmv (Al-Mohy-Higham) on the C4 graph: ms per fused Taylor term and its fraction of the HBM roofline
     (algorithmic bytes 4*nnz [pattern-only CSR] + 4*(n+1) + 32*n*q: read b, write b', read-modify-write f)."""
     from krylov_robustness_b200.graphs import rmat_graph_device
@@ -309,6 +329,9 @@ def bench_c4(kr, ctx):
            "peak_GBs": peak, "frac": bytes_term / (ms_term * 1e-3) / 1e9 / peak,
            "expmv_call_wall_s_incl_h2d_d2h": wall, "graph_gen_s": gen_s, "matrix_analysis_upload_s": upload_s,
            "gpu_launches": c1["launches"] - c0["launches"], "lambda_max_est": lam4}
+    rows = np.sort(np.random.default_rng(0).choice(n, min(n, 4096), replace=False))
+    outputs["c4_expmv_sample"] = f[rows]
+    outputs["c4_tscale"] = np.array([tscale])
     del M4, f, b
     return out
 
@@ -406,6 +429,7 @@ def run_ours(args):
     spmm_ms, spmm_launches = ctx.spmm_time(reset=True)
     ctx.set_timing(False)
     tr_value = float(tr_dev.item())
+    outputs = {"c3_trace": np.array([tr_value])}
 
     # ---- strong scaling of the headline (SURVEY.md 8e: the 512 probe columns SPLIT across the ranks)
     strong = None
@@ -450,6 +474,8 @@ def run_ours(args):
             return vals, (np.concatenate(its) if its else np.zeros(0))
         score_round(E[:64 * world])                       # warm-up (allocations, attribute setup)
         ms_edges, (vals, its) = timed(lambda: score_round(E), 1)
+        outputs["c5_edge_scores"] = vals
+        outputs["c5_candidates"] = E
         lo, hi = P.shard_bounds(E.shape[0])
         # edge roofline of SURVEY.md 8(d): matvec roofline / (2 * mean steps)
         b_mv = ((4.0 if pattern_only else 12.0) * nnz + 4.0 * (n + 1)) / 512 + 16.0 * n
@@ -502,28 +528,27 @@ def run_ours(args):
     for _ in range(1):
         step_e2e()
     h0 = ctx.counters()
-    ms_e2e, tr_e2e = timed(step_e2e, max(1, min(args.steps, 3)))
+    ms_e2e, tr_e2e = timed(step_e2e, args.steps)
     h1 = ctx.counters()
-    e2e_steps = max(1, min(args.steps, 3))
     step_e2e_sign()
     g0 = ctx.counters()
-    ms_e2e8, tr_e2e8 = timed(step_e2e_sign, e2e_steps)
+    ms_e2e8, tr_e2e8 = timed(step_e2e_sign, args.steps)
     g1 = ctx.counters()
 
     # ---- config C4: expmv Taylor path on R-MAT 2^24 nodes / 2^28 stored entries, 64 right-hand sides, normAm on the
     # device.  One GPU's worth of work (A replicated, columns would be split): measured on rank 0 when N == 1.
     secondary_c4 = None
     if rank == 0 and os.environ.get("KR_BENCH_C4", "1" if world == 1 else "0") != "0":
-        secondary_c4 = bench_c4(kr, ctx)
+        secondary_c4 = bench_c4(kr, ctx, outputs)
     # ---- config C2: gradient over all edges of the largest Transport road network (rank 0, N == 1)
     secondary_c2 = None
     if rank == 0 and os.environ.get("KR_BENCH_C2", "1" if world == 1 else "0") != "0":
-        secondary_c2 = bench_c2(kr, ctx)
+        secondary_c2 = bench_c2(kr, ctx, outputs)
 
     if rank == 0:
         mv_step = k * m * world
         value = mv_step * args.steps / (ms_dev * 1e-3)
-        e2e = mv_step * e2e_steps / (ms_e2e * 1e-3)
+        e2e = mv_step * args.steps / (ms_e2e * 1e-3)
         peak = peak_gbs()
         src = PEAK_SOURCE[0]
         # algorithmic bytes with the matrix as it is actually stored (pattern-only CSR: 4 B per nonzero)
@@ -550,13 +575,13 @@ def run_ours(args):
             "trace_estimate": tr_value, "lambda_scale": lam,
             "clocks": clocks, "numa": numa,
             "e2e": {"value": e2e, "unit": UNIT,
-                    "h2d_bytes_per_step": (h1["h2d_bytes"] - h0["h2d_bytes"]) // e2e_steps,
-                    "d2h_bytes_per_step": (h1["d2h_bytes"] - h0["d2h_bytes"]) // e2e_steps + 8,
-                    "ms_per_step": ms_e2e / e2e_steps, "trace_estimate": tr_e2e},
+                    "h2d_bytes_per_step": (h1["h2d_bytes"] - h0["h2d_bytes"]) // args.steps,
+                    "d2h_bytes_per_step": (h1["d2h_bytes"] - h0["d2h_bytes"]) // args.steps + 8,
+                    "ms_per_step": ms_e2e / args.steps, "trace_estimate": tr_e2e},
             # same call path with the probes handed over as int8 signs (kr_slq_trace_sign): 1/8 of the upload
-            "e2e_sign_probes": {"value": mv_step * e2e_steps / (ms_e2e8 * 1e-3), "unit": UNIT,
-                                "h2d_bytes_per_step": (g1["h2d_bytes"] - g0["h2d_bytes"]) // e2e_steps,
-                                "ms_per_step": ms_e2e8 / e2e_steps, "trace_estimate": tr_e2e8},
+            "e2e_sign_probes": {"value": mv_step * args.steps / (ms_e2e8 * 1e-3), "unit": UNIT,
+                                "h2d_bytes_per_step": (g1["h2d_bytes"] - g0["h2d_bytes"]) // args.steps,
+                                "ms_per_step": ms_e2e8 / args.steps, "trace_estimate": tr_e2e8},
             "gpu_launches": c1["launches"] - c0["launches"],
             "roofline": {"bound": "hbm", "kernel": "spmm_kernel<EpiDot> (CSR x %d-wide fp64 block + fused alpha dot)" % int(round(cols_per_launch)),
                          "columns_per_launch": cols_per_launch,
@@ -579,6 +604,8 @@ def run_ours(args):
                                        "of the same graph, %.1f s" % (m, cpu_dt)},
         }
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -588,10 +615,16 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every C3 arm")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed steps before the C3 timing (--impl ours runs at least 3)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed calls returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

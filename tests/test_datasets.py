@@ -1,5 +1,6 @@
 """datasets.py (MAT-file loading + the scripts' preprocessing) against the committed fixtures.  The reference's data
-files only exist in the build container (/root/reference); the preprocessing helpers are also tested stand-alone."""
+files are read from a checkout of the reference named by KR_REFERENCE_DIR; the preprocessing helpers are also tested
+stand-alone."""
 import os
 
 import numpy as np
@@ -8,7 +9,8 @@ import scipy.sparse as sp
 
 from conftest import load_graph
 
-REF = "/root/reference"
+REF = os.environ.get("KR_REFERENCE_DIR", "")
+needs_ref = pytest.mark.skipif(not (REF and os.path.isdir(REF)), reason="KR_REFERENCE_DIR names no checkout of the reference")
 
 
 def test_unweighted_preprocessing_on_a_toy_graph():
@@ -20,7 +22,7 @@ def test_unweighted_preprocessing_on_a_toy_graph():
     assert B.diagonal().sum() == 0 and set(B.data) == {1.0}
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference data files only exist in the build container")
+@needs_ref
 def test_loaders_reproduce_the_fixtures():
     from krylov_robustness_b200 import datasets as D
     for name, path in (("transport_Anaheim", "datasets_paper/Transport/Anaheim.mat"),
@@ -36,7 +38,7 @@ def test_loaders_reproduce_the_fixtures():
         assert A.shape == F.shape and abs(A - F).max() <= 1e-15
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference data files only exist in the build container")
+@needs_ref
 def test_v73_files_through_the_minimal_hdf5_reader():
     """CollegeMsg, Drugs, as_735 are MATLAB v7.3 (HDF5) files; the image has no HDF5 library, hdf5_min.py reads them.
     Two of them carry the symmetrised pattern a second time (variable W, written by a different code path of MATLAB):

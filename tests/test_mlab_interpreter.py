@@ -1,7 +1,7 @@
 """The MATLAB-subset interpreter (oracle/mlab) that executes the reference's own functions/*.m to pin parity.
 
 Two tiers, both CPU: language semantics on small snippets whose MATLAB results are known by definition of the
-language, and - where a checkout of the reference is present (this container; not the GPU box) - the reference's
+language, and - where KR_REFERENCE_DIR names a checkout of the reference - the reference's
 unmodified sources executed live: every file parses, the committed golden file is reproduced bit for bit, and the
 L1 recurrences agree with the oracle on fresh random inputs."""
 import io
@@ -19,9 +19,9 @@ from conftest import GOLDEN, ROOT, load_graph
 
 from oracle.mlab import Interpreter, MatlabError, Cell, Struct
 
-REFDIR = "/root/reference"
-has_ref = pytest.mark.skipif(not os.path.isdir(os.path.join(REFDIR, "functions")),
-                             reason="no checkout of the reference here (the GPU box): the committed goldens stand in")
+REFDIR = os.environ.get("KR_REFERENCE_DIR", "")
+has_ref = pytest.mark.skipif(not (REFDIR and os.path.isdir(os.path.join(REFDIR, "functions"))),
+                             reason="KR_REFERENCE_DIR names no checkout of the reference: the committed goldens stand in")
 
 
 def run(src, tmp_path, **ws):
@@ -242,9 +242,9 @@ def test_every_reference_function_file_parses():
 
 @has_ref
 def test_committed_goldens_are_what_the_reference_sources_produce():
-    """Re-runs scripts/make_reference_goldens.m over /root/reference/functions/*.m: bit-for-bit the committed file."""
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "scripts", "run_reference_goldens.py"), "--check"],
-                       capture_output=True, text=True, timeout=900)
+    """Re-runs scripts/make_reference_goldens.m over the reference's functions/*.m: bit-for-bit the committed file."""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "scripts", "run_reference_goldens.py"), "--refdir", REFDIR,
+                        "--check"], capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
     assert "reproduced bit for bit" in r.stdout
     prov = json.load(open(os.path.join(GOLDEN, "reference_golden.provenance.json")))
