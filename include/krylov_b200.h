@@ -149,8 +149,7 @@ int  kr_fun_update_fetch(kr_ctx* ctx, double* Xm, int64_t ldx, double* Um, int64
  * One single-vector Arnoldi space per distinct first index (:42, :86-110).  On a symmetric matrix a space whose vectors stay
  * on a small ball around its start node (road networks) is run whole by one CTA in shared memory (csrc/entries_local.cuh);
  * the others are advanced together by n x R SpMMs.  Same arithmetic (arnoldi_krylov.m:104-106), same iteration count.
- * Environment (debugging / A-B): KR_ENTRIES_LOCAL=0 dense batch only, KR_ENTRIES_LOCAL_TIER=t first budget tier,
- * KR_ENTRIES_LOCAL_SOLVE=2|1|0 projected solve by scaled Taylor (default) | tridiagonal QL | Jacobi, KR_ENTRIES_CHUNK_COLS=c columns per dense chunk. */
+ * Environment (testing): KR_ENTRIES_LOCAL=0 dense batch only, KR_ENTRIES_CHUNK_COLS=c columns per dense chunk. */
 int  kr_function_multiple_entries(kr_ctx* ctx, const kr_matrix* A, int64_t k, const int64_t* omega,
                                   int fun, double tol, int64_t it, double* X, int64_t* iter);
 /* [f,gr] = fun_and_grad_krylov_exp(X,A,Omega,eA,tol,it,debug)   functions/fun_and_grad_krylov_exp.m:1-113

@@ -254,7 +254,7 @@ int kr_matrix_set_edges(kr_matrix* A, int64_t count, const int64_t* ii, const in
         // The device keeps the stored CSR untouched and applies the few pending entries on the fly in the SpMM and
         // in the candidate-seed kernel (the greedy loop's only consumers): no host rebuild, no re-upload of A per
         // round.  Unsymmetric matrices (a transposed copy exists) and very long edit lists take the rebuild.
-        if (!A->symmetric || A->pending.size() > KR_MAX_PENDING || getenv("KR_SET_EDGES_REBUILD")) flush_pending(A);
+        if (!A->symmetric || A->pending.size() > KR_MAX_PENDING) flush_pending(A);
         else upload_pending(A);
         for (kr_matrix* P : A->peers)                // the same edit on every replica (a few hundred bytes each)
             if (kr_matrix_set_edges(P, count, ii, jj, v) != 0) fail(KR_ERR_CUDA, "replica on device %d: %s", P->ctx->device, kr_last_error());

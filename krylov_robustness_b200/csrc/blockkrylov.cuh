@@ -10,7 +10,6 @@
 //   the device; per Krylov step the host reads back a handful of scalars (one synchronisation).
 // No cuBLAS / cuSOLVER anywhere (round 1 used dgemm / geqrf / orgqr / syevd here).
 #pragma once
-#include <chrono>
 #include <memory>
 
 #include "dense.cuh"
@@ -64,25 +63,6 @@ inline bool is_symmetric(const HostMat& B) {
             if (B(i, j) != B(j, i)) return false;
     return B.rows == B.cols;
 }
-
-// ---- host-side phase timers of the wide-block path (KR_PROFILE_WIDE=1 prints them to stderr at the end of
-// fun_update / trace_fun_update; they synchronise the stream, so they are a diagnostic, not a product path)
-struct WideProf {
-    bool on = getenv("KR_PROFILE_WIDE") != nullptr;
-    double step = 0, fun = 0;
-    int n_step = 0, n_fun = 0, max_dim = 0;
-    static double now() {
-        return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count();
-    }
-    void report(const char* what) {
-        if (!on) return;
-        fprintf(stderr, "[kr wide] %s: krylov steps %d %.2f ms | f(Gm) evaluations %d %.2f ms (largest n %d)\n", what,
-                n_step, step, n_fun, fun, max_dim);
-        step = fun = 0;
-        n_step = n_fun = max_dim = 0;
-    }
-};
-inline WideProf& wide_prof() { static WideProf p; return p; }
 
 // ------------------------------------------------------------------------------------ small device kernels
 __global__ void add_inplace_kernel(double* __restrict__ a, const double* __restrict__ b, int64_t total) {
@@ -498,13 +478,10 @@ inline TfuResult trace_fun_update_general(kr_ctx* ctx, const kr_matrix* M, int64
     int64_t j = 0;
     DevBuf<double> SG, F;
     for (j = 1; j <= it; ++j) {
-        const double t0 = wide_prof().on ? WideProf::now() : 0.0;
         if (j > 1) krylov_step(st);
-        if (wide_prof().on) { KR_CUDA(cudaStreamSynchronize(ctx->stream)); wide_prof().step += WideProf::now() - t0; wide_prof().n_step++; }
         const int nn = (int)(j * rk);
         const size_t sz = (size_t)2 * nn * nn;
         if (SG.count < sz) { SG.reset(ctx, sz); F.reset(ctx, sz); }
-        const double t1 = wide_prof().on ? WideProf::now() : 0.0;
         KR_LAUNCH(ctx, assemble_proj_kernel, ew_grid(ctx, (int64_t)nn * nn), 256, 0, st->hblocks(), nn, ws.CmS.p, (int)rk, SG.p);
         for (int attempt = 0; attempt < 2; ++attempt) {
             ew.begin(ctx, attempt == 1);
@@ -515,7 +492,6 @@ inline TfuResult trace_fun_update_general(kr_ctx* ctx, const kr_matrix* M, int64
             sync_lucky(st);                                   // the step's only synchronisation
             if (ew.accept()) break;
         }
-        if (wide_prof().on) { wide_prof().fun += WideProf::now() - t1; wide_prof().n_fun++; wide_prof().max_dim = std::max(wide_prof().max_dim, nn); }
         out.lucky = st->lucky;
         bool done = false;
         if (j <= 2) Xstop[j - 1] = out.Xm;
@@ -526,7 +502,6 @@ inline TfuResult trace_fun_update_general(kr_ctx* ctx, const kr_matrix* M, int64
         if (done || st->lucky) break;
     }
     out.iter = std::min(j, it);
-    wide_prof().report("trace_fun_update");
     return out;
 }
 
@@ -584,9 +559,7 @@ inline FuInfo fun_update_general(kr_ctx* ctx, const kr_matrix* M, int64_t rk, co
     DevBuf<int> need(ctx, 1);
     int64_t j = 0;
     for (j = 1; j <= it; ++j) {
-        const double t0 = wide_prof().on ? WideProf::now() : 0.0;
         if (j > 1) krylov_step(st);
-        if (wide_prof().on) { KR_CUDA(cudaStreamSynchronize(ctx->stream)); wide_prof().step += WideProf::now() - t0; wide_prof().n_step++; }
         if (want_basis && 2 * st->vcols() >= n) {               // :85-90 dense fallback
             sync_lucky(st);
             dense_fallback(j, st->lucky);
@@ -595,7 +568,6 @@ inline FuInfo fun_update_general(kr_ctx* ctx, const kr_matrix* M, int64_t rk, co
         const int nn = (int)(j * rk);
         const size_t sz = (size_t)nn * nn;
         if (SG.count < 2 * sz) { SG.reset(ctx, 2 * sz); F.reset(ctx, 2 * sz); D.reset(ctx, sz); }
-        const double t1 = wide_prof().on ? WideProf::now() : 0.0;
         KR_LAUNCH(ctx, assemble_proj_kernel, ew_grid(ctx, (int64_t)sz), 256, 0, st->hblocks(), nn, ws.CmS.p, (int)rk, SG.p);
         Xs.emplace_back(ctx, sz);
         Xdim.push_back(nn);
@@ -619,7 +591,6 @@ inline FuInfo fun_update_general(kr_ctx* ctx, const kr_matrix* M, int64_t rk, co
             sync_lucky(st);                                   // the step's only synchronisation
             if (ew.accept()) break;
         }
-        if (wide_prof().on) { wide_prof().fun += WideProf::now() - t1; wide_prof().n_fun++; wide_prof().max_dim = std::max(wide_prof().max_dim, nn); }
         info.lucky = st->lucky;
         bool done = false;
         if (j > 2) {
@@ -640,7 +611,6 @@ inline FuInfo fun_update_general(kr_ctx* ctx, const kr_matrix* M, int64_t rk, co
     // Um(:, 1:size(Xm,1))  (:137) - for Lanczos this is the 2-block window, as in the reference
     res.Um = std::move(st->V);
     KR_CUDA(cudaStreamSynchronize(ctx->stream));
-    wide_prof().report("fun_update");
     return info;
 }
 
@@ -842,8 +812,7 @@ inline CentralityInfo leading_vector_dev(kr_ctx* ctx, const kr_matrix* M, int mo
     if (n == 0) return info;
     if (mode == 1 && !M->symmetric) fail(KR_ERR_UNSUPPORTED, "compute_centrality 'pr': the device path expects a symmetric A");
     DevBuf<double> x(ctx, n), y(ctx, n), z(ctx, n), sc(ctx, 4), part(ctx, VEC_RED_CTAS);
-    static const int64_t small_nnz = [] { const char* e = getenv("KR_NORMEST_SMALL_NNZ"); return e ? atoll(e) : (int64_t)400000; }();
-    if (M->dev.nnz <= small_nnz) {
+    if (M->dev.nnz <= CSR_L2_RESIDENT_NNZ) {
         KR_LAUNCH(ctx, power_iteration_small_kernel, 1, 1024, 0, M->dev.view(), mode, tol, (int)std::min<int64_t>(maxit, 1 << 30), x.p, y.p, z.p, sc.p);
         double h[2];
         sc.download(h, 2);
@@ -890,8 +859,7 @@ inline void normest_dev(kr_ctx* ctx, const kr_matrix* M, double tol, double* est
     const int64_t n = M->dev.n;
     if (n == 0) { *est = 0; *count = 0; return; }
     DevBuf<double> x(ctx, n), sx(ctx, n), part(ctx, VEC_RED_CTAS), sc(ctx, 4);
-    static const int64_t small_nnz = [] { const char* e = getenv("KR_NORMEST_SMALL_NNZ"); return e ? atoll(e) : (int64_t)400000; }();
-    if (M->dev.nnz <= small_nnz) {
+    if (M->dev.nnz <= CSR_L2_RESIDENT_NNZ) {
         KR_LAUNCH(ctx, normest_small_kernel, 1, 1024, 0, M->dev.view(), M->T().view(), tol, x.p, sx.p, sc.p);
         double h[3];
         sc.download(h, 3);

@@ -64,6 +64,9 @@ struct CsrDevView {
 constexpr int SPMM_CAP = KR_SPMM_CAP;             // nonzeros staged in shared memory per multi-row tile
 constexpr int SPMM_MAX_ROWS = KR_SPMM_MAX_ROWS;   // rows per tile
 constexpr int SPMM_LONG_ROW = 1024;   // rows at least this long are processed by a whole CTA
+// Stored entries up to which a CSR (4-12 B per entry) and a few n-vectors stay L2-resident: there the one-CTA paths
+// (pair_small_kernel, the single-CTA power iterations of leading_vector_dev and normest_dev) replace launch-bound loops.
+constexpr int64_t CSR_L2_RESIDENT_NNZ = 400000;
 
 struct CsrDev {
     int64_t n = 0, nnz = 0;

@@ -7,7 +7,7 @@
 //     so the local numbering - and with it every summation order - is deterministic),
 //   * local index order = BFS order, so basis vector l is stored with |ball(l)| entries only (a triangular arena),
 //   * w = A v_j by rows in stored CSR order, CGS2 + the third pass of arnoldi_krylov.m:104-106 (all inner products of
-//     a pass before its update, as the reference), the projected solve + lag-3 stop of entries_project_step,
+//     a pass before its update, as the reference), the projected solve by one warp + the lag-3 stop of entries_stop_test,
 //   * the requested entries f(A)(h, j2) = sum_l V_l(j2) x_l straight from the arena.
 // Columns are handed out by a ticket counter.  A column whose ball outgrows the CTA's budget is flagged and run again with
 // the next budget tier; one that outgrows the last tier (or that has not stopped after EL_IT steps while the caller allows
@@ -37,8 +37,6 @@ struct EntriesLocalArgs {
     int* flag;                       // [R] nonzero = not handled here (1: ball outgrew the budget, 2: step limit of this path)
     int* ticket;
     int R, itl, it_is_cap, fun;      // itl = min(it, EL_IT); it_is_cap: it <= EL_IT (running out of steps is final)
-    int use_ql;                      // projected solve: 2 = scaled Taylor of e^{+-T} e1 by one warp (QL when ||T|| is large),
-                                     // 1 = tridiagonal QL by one warp, 0 = the dense path's Jacobi
     int maxn, hcap, hshift, arena;   // budget (hshift = 32 - log2 hcap)
     const int* sel;                  // columns to process (null: all of 0..R-1)
     int nsel;
@@ -57,11 +55,9 @@ __device__ __forceinline__ int el_lookup(const int* keys, const int* vals, int g
     }
 }
 
-__host__ __device__ inline int el_scratch_doubles(int itl, int use_ql) {
-    return use_ql ? itl * (EL_IT + 1) + itl : 2 * itl * (itl | 1) + itl;
-}
 constexpr int EL_LDQ = EL_IT + 1;   // odd: the lanes' rows of Q fall into different banks
 static_assert(EL_IT <= 32 && (EL_LDQ & 1) == 1, "one lane per row of Q");
+__host__ __device__ inline int el_scratch_doubles(int itl) { return itl * EL_LDQ + itl; }   // Q (itl x EL_LDQ) + x
 
 // x = f(T) e1 for the symmetric tridiagonal part T of the projection (diagonal H(i,i), off-diagonal the mean of H(i+1,i)
 // and H(i,i+1)): implicit QL with eigenvector accumulation (EISPACK tql2) run by ONE warp without any barrier - every
@@ -208,8 +204,9 @@ entries_local_kernel(CsrDevView A, EntriesLocalArgs a) {
     double* arena = dyn;
     double* Hl = arena + a.arena;                        // it1 columns of it1 + 1
     double* ring = Hl + it1 * (it1 + 1);                  // 4 x it1
-    double* scratch = ring + 4 * it1;                     // Jacobi: 2 jj (jj|1) + jj for jj <= itl; QL: Q (itl x EL_LDQ) + x
-    int* keys = reinterpret_cast<int*>(scratch + el_scratch_doubles(a.itl, a.use_ql));
+    double* Q = ring + 4 * it1;                          // QL fallback: itl x EL_LDQ
+    double* fx = Q + a.itl * EL_LDQ;                     // f(T) e1 of the latest step
+    int* keys = reinterpret_cast<int*>(Q + el_scratch_doubles(a.itl));
     int* vals = keys + a.hcap;
     int* L = vals + a.hcap;                              // global ids in local order
     int* rs = L + a.maxn;                                // first stored nonzero of the node's row
@@ -354,17 +351,9 @@ entries_local_kernel(CsrDevView A, EntriesLocalArgs a) {
             }
             // ---- projected problem and stopping test
             const int jj = j + 1;
-            if (a.use_ql) {
-                if (warp == 0) {
-                    double* xs = scratch + a.itl * EL_LDQ;
-                    if (a.use_ql != 2 || !warp_tridiag_fx_taylor(Hl, it1, jj, a.fun, xs))
-                        warp_tridiag_fx(Hl, it1, jj, a.fun, scratch, xs);
-                }
-                __syncthreads();
-                done = entries_stop_test(scratch + a.itl * EL_LDQ, it1, jj, a.tol, ring, &sh);
-            } else {
-                done = entries_project_step(Hl, it1, jj, a.fun, a.tol, ring, scratch, &sh);
-            }
+            if (warp == 0 && !warp_tridiag_fx_taylor(Hl, it1, jj, a.fun, fx)) warp_tridiag_fx(Hl, it1, jj, a.fun, Q, fx);
+            __syncthreads();
+            done = entries_stop_test(fx, it1, jj, a.tol, ring, &sh);
             nsteps = jj;
             __syncthreads();
             if (done) break;
@@ -374,14 +363,13 @@ entries_local_kernel(CsrDevView A, EntriesLocalArgs a) {
             continue;
         }
         // ---- entries: X[p] = sum_{l < nsteps} V_l(j2) x_l     (function_multiple_entries.m:162-164)
-        const double* x = a.use_ql ? scratch + a.itl * EL_LDQ : scratch + 2 * nsteps * (nsteps | 1);
         for (int q = a.pair_begin[c] + tid; q < a.pair_begin[c + 1]; q += JAC_THREADS) {
             const int p = a.pair_list[q];
             const int li = el_lookup(keys, vals, (int)(a.j2[p] - 1), a.hshift, hmask);
             double s = 0.0;
             if (li >= 0)
                 for (int l = 0; l < nsteps; ++l)
-                    if (li < len[l]) s += arena[off[l] + li] * x[l];
+                    if (li < len[l]) s += arena[off[l] + li] * fx[l];
             a.X[p] = s;
         }
         if (tid == 0) { a.flag[c] = 0; a.steps[c] = nsteps; }
@@ -393,9 +381,9 @@ struct EntriesLocalResult {
     std::vector<int> steps, flag;    // [R]
 };
 
-inline size_t entries_local_smem(int itl, int use_ql, const EntriesLocalBudget& b) {
+inline size_t entries_local_smem(int itl, const EntriesLocalBudget& b) {
     const int it1 = itl + 1;
-    return (size_t)(b.arena + it1 * (it1 + 1) + 4 * it1 + el_scratch_doubles(itl, use_ql)) * sizeof(double) +
+    return (size_t)(b.arena + it1 * (it1 + 1) + 4 * it1 + el_scratch_doubles(itl)) * sizeof(double) +
            (size_t)(2 * b.hcap + 3 * b.maxn) * sizeof(int);
 }
 
@@ -435,19 +423,13 @@ inline EntriesLocalResult entries_local_run(kr_ctx* ctx, const kr_matrix* M, con
     a.it_is_cap = it <= EL_IT;
     a.fun = fun;
     a.tol = tol;
-    a.use_ql = 2;
-    if (const char* e = getenv("KR_ENTRIES_LOCAL_SOLVE")) a.use_ql = std::min(std::max(atoi(e), 0), 2);     // A/B switch
-    if (const char* e = getenv("KR_ENTRIES_LOCAL_JACOBI")) if (atoi(e) != 0) a.use_ql = 0;
     static bool attr_set[64] = {};
     if (first_use_on_device(attr_set, ctx->device))
         KR_CUDA(cudaFuncSetAttribute(entries_local_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)std::max(entries_local_smem(EL_IT, 0, EL_TIERS[EL_NTIERS - 1]),
-                                                   entries_local_smem(EL_IT, 1, EL_TIERS[EL_NTIERS - 1]))));
-    int first_tier = 0;
-    if (const char* e = getenv("KR_ENTRIES_LOCAL_TIER")) first_tier = std::min(std::max(atoi(e), 0), EL_NTIERS - 1);   // A/B switch
+                                     (int)entries_local_smem(EL_IT, EL_TIERS[EL_NTIERS - 1])));
     DevBuf<int> dsel;
     std::vector<int> sel;                                   // empty: all columns
-    for (int tier = first_tier; tier < EL_NTIERS; ++tier) {
+    for (int tier = 0; tier < EL_NTIERS; ++tier) {
         const EntriesLocalBudget& b = EL_TIERS[tier];
         a.maxn = b.maxn;
         a.hcap = b.hcap;
@@ -458,7 +440,7 @@ inline EntriesLocalResult entries_local_run(kr_ctx* ctx, const kr_matrix* M, con
         a.sel = sel.empty() ? nullptr : dsel.p;
         a.nsel = (int)sel.size();
         const int todo = sel.empty() ? R : (int)sel.size();
-        const size_t smem = entries_local_smem(a.itl, a.use_ql, b);
+        const size_t smem = entries_local_smem(a.itl, b);
         const int per_sm = std::max(1, (int)((size_t)228 * 1024 / (smem + 4096 + 1024)));      // + static + the per-CTA reserve
         const int ctas = (int)std::min<int64_t>(todo, (int64_t)ctx->num_sms * per_sm);
         KR_CUDA(cudaMemsetAsync(a.ticket, 0, sizeof(int), ctx->stream));

@@ -86,14 +86,8 @@ __device__ __forceinline__ void mtm2(const double* A, const double* B, double* C
     C[0] = c0; C[1] = c1; C[2] = c2; C[3] = c3;
 }
 
-inline int pair_eig_jacobi() {
-    const char* e = getenv("KR_PAIR_EIG_JACOBI");
-    return (e && atoi(e) != 0) ? 1 : 0;
-}
-
 struct PairState {
     int nslots, it, fun;
-    int eig_jacobi;   // A/B switch (KR_PAIR_EIG_JACOBI=1): projected eigenvalues by cyclic Jacobi instead of tridiagonal multisection
     double tol, b_off;
     // ---- per slot
     long long* cand;  // [nslots] index of the candidate in the caller's list, -1 = idle
@@ -372,7 +366,7 @@ __device__ inline void pair_qr_from_gram(double g11, double g12, double g22, dou
 // (shared or global), nn = 2j.
 template <int NT>
 __device__ double pair_projected_trace(const double* Hd, const double* Hs, const double* Hr, int j, double b_off, int fun,
-                                       double* work, JacobiShared* sh, bool use_jacobi = false) {
+                                       double* work, JacobiShared* sh) {
     const int nn = 2 * j, lda = nn | 1;
     double* G = work;
     double* tG = G + nn * lda;
@@ -395,7 +389,7 @@ __device__ double pair_projected_trace(const double* Hd, const double* Hs, const
         tG[r + c * lda] = v + cm;
     }
     __syncthreads();
-    if (nn <= MS_MAX_N && !use_jacobi) {
+    if (nn <= MS_MAX_N) {
         // LAPACK's route (tridiagonalise + tridiagonal eigenvalues): two warps reduce one matrix each, then all threads
         // bracket all eigenvalues of both by multisection on Sturm counts (smalldense.cuh)
         __shared__ double ms_work[2][6 * MS_MAX_N];
@@ -448,7 +442,7 @@ pair_step_kernel(PairState st, const double* __restrict__ G3, double* __restrict
     }
     __syncthreads();
     double* work = gscratch ? gscratch + (int64_t)h * gscratch_stride : dyn;
-    const double Xm = pair_projected_trace<JAC_THREADS>(Hd, Hs, Hr, j, st.b_off, st.fun, work, &sh, st.eig_jacobi != 0);
+    const double Xm = pair_projected_trace<JAC_THREADS>(Hd, Hs, Hr, j, st.b_off, st.fun, work, &sh);
     if (threadIdx.x == 0) {
         bool done = false;
         double* Xs = st.Xstop + h * 2;
@@ -516,7 +510,6 @@ inline void pairs_run(kr_ctx* ctx, const kr_matrix* M, const int64_t* Ei, const 
     istate.zero();
     PairState st;
     st.nslots = ns; st.it = it; st.fun = fun; st.tol = tol; st.b_off = b_off;
-    st.eig_jacobi = pair_eig_jacobi();
     double* d = dstate.p;
     st.Tp = d; d += ns * 4;
     st.Tc = d; d += ns * 4;

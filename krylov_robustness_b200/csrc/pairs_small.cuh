@@ -30,8 +30,6 @@ struct PairSmallArgs {
     const int* ei;                      // [np] 0-based end points
     const int* ej;
     int np, it, fun;
-    int eig_jacobi;                     // A/B switch, see PairState
-    int debug_skip_eig;                 // timing experiments only (KR_PS_DEBUG_SKIP_EIG=steps): no eigen-solves, fixed step count
     double tol, b_off;
     double2* ws;                        // [ctas][3][n]
     double* hbuf;                       // [ctas][3][it][4]: Hd, Hs, Hr
@@ -361,12 +359,10 @@ pair_small_kernel(PairSmallArgs a) {
             }
             __syncthreads();
             double* work = 2 * jj <= PS_SMEM_NN ? dyn : gwork;
-            const double Xm = a.debug_skip_eig ? 0.0 : pair_projected_trace<PS_THREADS>(Hd, Hs, Hr, jj, a.b_off, a.fun, work, &sh, a.eig_jacobi != 0);
+            const double Xm = pair_projected_trace<PS_THREADS>(Hd, Hs, Hr, jj, a.b_off, a.fun, work, &sh);
             if (tid == 0) {
                 bool done = false;
-                if (a.debug_skip_eig) {
-                    done = jj >= a.debug_skip_eig;
-                } else if (jj <= 2) {
+                if (jj <= 2) {
                     Xs[jj - 1] = Xm;
                 } else {
                     const double err = fabs(Xm - Xs[0]);                              // trace_fun_update.m:104-118
@@ -398,17 +394,13 @@ pair_small_kernel(PairSmallArgs a) {
     }
 }
 
-inline int64_t pair_small_nnz_limit() {
-    static const int64_t v = [] { const char* e = getenv("KR_PAIR_SMALL_NNZ"); return e ? atoll(e) : (int64_t)400000; }();
-    return v;
-}
 // Where the single-launch path wins (profiles/r02n_time_pairs_small_*.jsonl): the CSR and one CTA's three n x 2 blocks
 // must stay cache-resident, and with more candidates than SMs a CTA's latency-bound row loops are no longer hidden
 // by other CTAs - there the batched pipeline catches up (n = 13 947, 250 candidates: 3.6 vs 3.4 ms).
 inline bool use_pairs_small(const kr_ctx* ctx, const kr_matrix* M, int64_t np) {
     if (getenv("KR_PAIR_SLOTS")) return false;                   // test hook of the batched pipeline
     const int64_t n = M->dev.n;
-    if (M->dev.nnz > pair_small_nnz_limit() || n > 20000) return false;
+    if (M->dev.nnz > CSR_L2_RESIDENT_NNZ || n > 20000) return false;
     return np <= ctx->num_sms || n <= 8192;
 }
 
@@ -453,8 +445,6 @@ inline void pairs_small_run(kr_ctx* ctx, const kr_matrix* M, const int64_t* Ei, 
     DevBuf<int> rl(ctx, (size_t)np);
     a.ei = de.p; a.ej = de.p + np; a.ticket = de.p + 2 * np;
     a.np = (int)np; a.it = it; a.fun = fun; a.tol = tol; a.b_off = b_off;
-    a.eig_jacobi = pair_eig_jacobi();
-    a.debug_skip_eig = getenv("KR_PS_DEBUG_SKIP_EIG") ? atoi(getenv("KR_PS_DEBUG_SKIP_EIG")) : 0;
     a.ws = ws.p; a.hbuf = hbuf.p;
     a.res_Xm = rx.p; a.res_iter = ri.p; a.res_lucky = rl.p;
     KR_LAUNCH(ctx, pair_small_kernel, ctas, PS_THREADS, PS_DYN_SMEM, a);

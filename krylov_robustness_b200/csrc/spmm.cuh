@@ -16,8 +16,6 @@
 //
 // HBM roofline (DESIGN.md): algorithmic bytes per launch = 12*nnz + 4*(n+1) + 16*n*k.
 #pragma once
-#include <type_traits>
-
 #include "csr.cuh"
 
 namespace kr {
@@ -49,8 +47,8 @@ struct PanelBlock {                // non-owning view of a panel-major block
 
 // A lane of the SpMM handles CPL consecutive columns of a row-tile with ONE load:
 //   CPL = 2: 128-bit gathers, 8 lanes per row-tile (the candidate-pair epilogue: one candidate per lane)
-//   CPL = 4: 256-bit gathers (LDG.E.256), 4 lanes per row-tile - half the load / address / index
-//            instructions per byte; the sustained SLQ pass is power-capped, so instructions per byte matter.
+//   CPL = 4: 256-bit gathers (LDG.E.256), 4 lanes per row-tile (EpiPlain, EpiDot, EpiTaylor) - half the load /
+//            address / index instructions per byte; the sustained SLQ pass is power-capped, so instructions per byte matter.
 template <int CPL>
 struct Vec {
     double v[CPL];
@@ -78,30 +76,14 @@ __device__ __forceinline__ Vec<4> ld_x<4>(const double* p) {
         : "=d"(r.v[0]), "=d"(r.v[1]), "=d"(r.v[2]), "=d"(r.v[3]) : "l"(p));
     return r;
 }
-template <int CPL>
-__device__ __forceinline__ Vec<CPL> ld_row(const double* p);        // row-local operand (plain cached load)
-template <>
-__device__ __forceinline__ Vec<2> ld_row<2>(const double* p) {
-    const double2 t = *reinterpret_cast<const double2*>(p);
-    Vec<2> r;
-    r.v[0] = t.x; r.v[1] = t.y;
-    return r;
-}
-template <>
-__device__ __forceinline__ Vec<4> ld_row<4>(const double* p) {
+__device__ __forceinline__ Vec<4> ld_row(const double* p) {           // row-local operand (plain cached load)
     Vec<4> r;
     asm volatile("ld.global.v4.f64 {%0, %1, %2, %3}, [%4];"
                  : "=d"(r.v[0]), "=d"(r.v[1]), "=d"(r.v[2]), "=d"(r.v[3]) : "l"(p));
     return r;
 }
-__device__ __forceinline__ void st_row(double* p, const Vec<2>& a) {
-    *reinterpret_cast<double2*>(p) = make_double2(a.v[0], a.v[1]);
-}
 __device__ __forceinline__ void st_row(double* p, const Vec<4>& a) {
     asm volatile("st.global.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(p), "d"(a.v[0]), "d"(a.v[1]), "d"(a.v[2]), "d"(a.v[3]) : "memory");
-}
-__device__ __forceinline__ void st_stream(double* p, const Vec<2>& a) {
-    __stcs(reinterpret_cast<double2*>(p), make_double2(a.v[0], a.v[1]));
 }
 __device__ __forceinline__ void st_stream(double* p, const Vec<4>& a) {
     asm volatile("st.global.cs.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(p), "d"(a.v[0]), "d"(a.v[1]), "d"(a.v[2]), "d"(a.v[3]) : "memory");
@@ -160,9 +142,8 @@ __device__ __forceinline__ void cta_reduce_by_sub(double (&v)[NV], double* smem)
 // (columns sub*CPL .. sub*CPL + CPL - 1 of the panel).
 
 // Y = alpha * (A*X - mu*X)
-template <int CPL_>
-struct EpiPlainT {
-    static constexpr int CPL = CPL_;
+struct EpiPlain {
+    static constexpr int CPL = 4;
     double* __restrict__ Y;        // panel base
     const double* __restrict__ X;  // panel base (for the shift term)
     double alpha, mu;
@@ -170,18 +151,14 @@ struct EpiPlainT {
         Y += q * stride;
         X += q * stride;
     }
-    // Row-local operands: with 128-bit lanes they are loaded before the gathers (latency hidden behind them); with
-    // 256-bit lanes the 4 x 32-byte gathers in flight need the registers, so pre() only pulls the line towards
-    // the SM and row() loads it afterwards.
+    // Row-local operands: the 4 x 32-byte gathers in flight need the registers, so pre() only pulls the line
+    // towards the SM and row() loads it afterwards.
     Vec<CPL> xr;
     __device__ __forceinline__ void pre(int r, int sub) {
-        if (mu != 0.0) {
-            if (CPL == 2) xr = ld_row<CPL>(X + (int64_t)r * PW + sub * CPL);
-            else if (sub == 0) prefetch_l1(X + (int64_t)r * PW);
-        }
+        if (mu != 0.0 && sub == 0) prefetch_l1(X + (int64_t)r * PW);
     }
     __device__ __forceinline__ void row(int r, int sub, Vec<CPL> y, unsigned) {
-        if (CPL != 2 && mu != 0.0) xr = ld_row<CPL>(X + (int64_t)r * PW + sub * CPL);
+        if (mu != 0.0) xr = ld_row(X + (int64_t)r * PW + sub * CPL);
 #pragma unroll
         for (int i = 0; i < CPL; ++i) {
             if (mu != 0.0) y.v[i] -= mu * xr.v[i];
@@ -193,9 +170,8 @@ struct EpiPlainT {
 };
 
 // Y = A*X and partial[tile][col] = sum_rows X(r,col) * Y(r,col)      (Lanczos alpha, SLQ path)
-template <int CPL_>
-struct EpiDotT {
-    static constexpr int CPL = CPL_;
+struct EpiDot {
+    static constexpr int CPL = 4;
     double* __restrict__ Y;
     const double* __restrict__ X;
     double* __restrict__ partial;  // [ntiles][panels*PW]
@@ -209,11 +185,10 @@ struct EpiDotT {
     }
     Vec<CPL> xr;
     __device__ __forceinline__ void pre(int r, int sub) {
-        if (CPL == 2) xr = ld_row<CPL>(X + (int64_t)r * PW + sub * CPL);
-        else if (sub == 0) prefetch_l1(X + (int64_t)r * PW);
+        if (sub == 0) prefetch_l1(X + (int64_t)r * PW);
     }
     __device__ __forceinline__ void row(int r, int sub, Vec<CPL> y, unsigned) {
-        if (CPL != 2) xr = ld_row<CPL>(X + (int64_t)r * PW + sub * CPL);      // (a non-volatile load here: no gain, profiles/r02aj_*)
+        xr = ld_row(X + (int64_t)r * PW + sub * CPL);      // (a non-volatile load here: no gain, profiles/r02aj_*)
 #pragma unroll
         for (int i = 0; i < CPL; ++i) acc[i] += xr.v[i] * y.v[i];
         st_stream(Y + (int64_t)r * PW + sub * CPL, y);
@@ -305,9 +280,8 @@ __device__ __forceinline__ void taylor_decide(TaylorCtl* ctl, double c2, double 
 //  * several panels: rowabs_b[panel][r] / rowabs_f[panel][r] are written and reduced by
 //    taylor_norms_ctl_kernel (expmv.cuh) - two launches per term.
 // Every launch returns immediately once *done != 0.
-template <int CPL_>
-struct EpiTaylorT {
-    static constexpr int CPL = CPL_;
+struct EpiTaylor {
+    static constexpr int CPL = 4;
     double* __restrict__ Bn;       // output b' panel
     const double* __restrict__ Bo; // input b panel (== X)
     double* __restrict__ F;        // f panel (read-modify-write)
@@ -330,21 +304,15 @@ struct EpiTaylorT {
     }
     Vec<CPL> xr, fr;
     __device__ __forceinline__ void pre(int r, int sub) {
-        const int64_t o = (int64_t)r * PW + sub * CPL;
-        if (CPL == 2) {
-            if (mu != 0.0) xr = ld_row<CPL>(Bo + o);
-            fr = ld_row<CPL>(F + o);
-        } else if (sub == 0) {
+        if (sub == 0) {
             if (mu != 0.0) prefetch_l1(Bo + (int64_t)r * PW);
             prefetch_l1(F + (int64_t)r * PW);
         }
     }
     __device__ __forceinline__ void row(int r, int sub, Vec<CPL> y, unsigned m) {
         const int64_t o = (int64_t)r * PW + sub * CPL;
-        if (CPL != 2) {
-            if (mu != 0.0) xr = ld_row<CPL>(Bo + o);
-            fr = ld_row<CPL>(F + o);
-        }
+        if (mu != 0.0) xr = ld_row(Bo + o);
+        fr = ld_row(F + o);
         Vec<CPL> f = fr;
         double ab = 0.0, af = 0.0;
 #pragma unroll
@@ -400,30 +368,6 @@ struct EpiTaylorT {
                 __threadfence();
             }
         }
-    }
-};
-
-// the lane width is a launch-time choice (KR_SPMM_CPL, default 4): callers fill the CPL = 2 flavour and
-// launch_spmm converts (same fields)
-using EpiPlain = EpiPlainT<2>;
-using EpiDot = EpiDotT<2>;
-using EpiTaylor = EpiTaylorT<2>;
-template <class Epi> struct WideEpi { using type = Epi; static type make(const Epi& e) { return e; } };
-template <> struct WideEpi<EpiPlain> {
-    using type = EpiPlainT<4>;
-    static type make(const EpiPlain& e) { type w; w.Y = e.Y; w.X = e.X; w.alpha = e.alpha; w.mu = e.mu; return w; }
-};
-template <> struct WideEpi<EpiDot> {
-    using type = EpiDotT<4>;
-    static type make(const EpiDot& e) { type w; w.Y = e.Y; w.X = e.X; w.partial = e.partial; w.total_cols = e.total_cols; return w; }
-};
-template <> struct WideEpi<EpiTaylor> {
-    using type = EpiTaylorT<4>;
-    static type make(const EpiTaylor& e) {
-        type w;
-        w.Bn = e.Bn; w.Bo = e.Bo; w.F = e.F; w.rab = e.rab; w.raf = e.raf; w.coef = e.coef; w.mu = e.mu;
-        w.ctl = e.ctl; w.total_ctas = e.total_ctas; w.full_term = e.full_term; w.tol = e.tol;
-        return w;
     }
 };
 
@@ -683,16 +627,13 @@ inline void launch_spmm_impl(kr_ctx* ctx, const CsrDev& A, const double* X, int 
     }
 }
 
+// independent gathers per lane and round: U2 for the 128-bit lanes (CPL = 2), U4 for the 256-bit lanes (CPL = 4)
 #ifndef KR_SPMM_U2
 #define KR_SPMM_U2 8
 #endif
 #ifndef KR_SPMM_U4
 #define KR_SPMM_U4 4
 #endif
-inline int spmm_lane_width() {
-    static const int w = [] { const char* e = getenv("KR_SPMM_CPL"); return (e && atoi(e) == 2) ? 2 : 4; }();
-    return w;
-}
 
 // Host-side launcher.  Epilogues carry panel-0 pointers; init() advances them to the CTA's panel.
 template <class Epi>
@@ -704,13 +645,7 @@ inline void launch_spmm(kr_ctx* ctx, const CsrDev& A, const double* X, int panel
         ctx->timing_events(&e0, &e1);
         KR_CUDA(cudaEventRecord(e0, ctx->stream));
     }
-    using Wide = WideEpi<Epi>;
-    if constexpr (!std::is_same<typename Wide::type, Epi>::value) {
-        if (spmm_lane_width() == 4) launch_spmm_impl<typename Wide::type, KR_SPMM_U4>(ctx, A, X, panels, Wide::make(epi), done, panel_active);
-        else launch_spmm_impl<Epi, KR_SPMM_U2>(ctx, A, X, panels, epi, done, panel_active);
-    } else {
-        launch_spmm_impl<Epi, KR_SPMM_U2>(ctx, A, X, panels, epi, done, panel_active);
-    }
+    launch_spmm_impl<Epi, Epi::CPL == 4 ? KR_SPMM_U4 : KR_SPMM_U2>(ctx, A, X, panels, epi, done, panel_active);
     check_launch(ctx, "spmm_kernel");
     if (ctx->timing) {
         KR_CUDA(cudaEventRecord(e1, ctx->stream));

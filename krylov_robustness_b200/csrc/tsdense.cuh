@@ -601,11 +601,6 @@ struct ThinQrWork {
     int64_t fallbacks = 0, calls = 0;
 };
 
-inline bool thin_qr_use_cholqr() {
-    static const bool v = [] { const char* e = getenv("KR_QR_HOUSEHOLDER"); return !(e && atoi(e) != 0); }();
-    return v;
-}
-
 // W (n x bs block given as one PanelBuf) <- Q of qr(W, 0) with LAPACK's sign conventions; work.hqr.st.R <- R.
 // Synchronises once (the breakdown flag decides between the two routes on the host).
 inline void thin_qr(kr_ctx* ctx, PanelBuf& Wb, int bs, ThinQrWork& work) {
@@ -613,7 +608,7 @@ inline void thin_qr(kr_ctx* ctx, PanelBuf& Wb, int bs, ThinQrWork& work) {
     PanelList W;
     W.add(Wb);
     work.calls += 1;
-    if (!thin_qr_use_cholqr() || n < bs || bs > CQ_MAXB) {
+    if (n < bs || bs > CQ_MAXB) {
         hqr_thin(ctx, W, n, bs, work.hqr);
         return;
     }

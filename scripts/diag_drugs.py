@@ -24,8 +24,3 @@ for h in np.argsort(-rel)[:8]:
     U, B = edge_UB(n, int(i), int(j), -1.0)
     xs, its, _ = kr.trace_fun_update(M, U, B, tol, 100, 0, "exp")
     print("   single-call path:", xs, its, abs(xs - ox[h]) / abs(ox[h]))
-import os
-for flag in ("KR_PAIR_EIG_JACOBI",):
-    os.environ[flag] = "1"
-    x2, it2, _ = kr.trace_fun_update_edges(M, E, -1.0, tol, 100, "exp")
-    print(flag, "max rel", (np.abs(x2 - ox) / np.abs(ox)).max())

@@ -1,5 +1,5 @@
 """One fun_and_grad_krylov_fun callback of the weighted experiments (30 modifiable edges) on a small graph: the call
-the launch list / KR_PROFILE_WIDE breakdown of scripts/gpu_r02_s.sh is taken from."""
+the launch list of scripts/gpu_r02_s.sh is taken from."""
 import os
 import sys
 import time

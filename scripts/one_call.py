@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""One call of one entry point on one of the reference's graphs (for ncu launch lists / KR_PROFILE_WIDE):
+"""One call of one entry point on one of the reference's graphs (for launch lists):
   python scripts/one_call.py fun_and_grad|tfu_rank2|edges250|centrality|normest|tfu_set [graph]"""
 import os
 import sys

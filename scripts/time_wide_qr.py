@@ -1,6 +1,5 @@
-"""A/B of the thin QR inside the wide-block path on a LARGE graph: trace_fun_update with a rank-32 update (an edge set,
-Tests/test_unweighted_break.m:94-95 shape) on a power-law graph with n = 200 000; KR_QR_HOUSEHOLDER=1 forces the
-Householder passes of round 2's first version."""
+"""Time of the wide-block path, thin QR included, on a LARGE graph: trace_fun_update with a rank-32 update (an edge set,
+Tests/test_unweighted_break.m:94-95 shape) on a power-law graph with n = 200 000."""
 import json
 import os
 import sys
@@ -30,5 +29,5 @@ l0 = M.ctx.counters()["launches"]
 t0 = time.perf_counter()
 x, it, lucky = kr.trace_fun_update(M, U, B, tol, 100)
 dt = time.perf_counter() - t0
-print(json.dumps({"n": n, "rk": 32, "householder_only": os.environ.get("KR_QR_HOUSEHOLDER", "0"), "ms": dt * 1e3, "steps": int(it),
+print(json.dumps({"n": n, "rk": 32, "ms": dt * 1e3, "steps": int(it),
                   "launches": M.ctx.counters()["launches"] - l0, "Xm": float(x)}))
