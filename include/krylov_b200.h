@@ -61,6 +61,9 @@ void* kr_ctx_stream(kr_ctx* ctx);     /* cudaStream_t the library launches on */
 int  kr_matrix_create(kr_ctx* ctx, int64_t n, int64_t nnz, const int64_t* row_ptr,
                       const int64_t* col_idx, const double* val, kr_matrix** out);
 void kr_matrix_destroy(kr_matrix* A);
+/* n, nnz, symmetric and nonnegative describe A with every kr_matrix_set_edges edit applied, pending or folded;
+ * asking folds nothing in.  pattern_only describes the storage: set when every stored value is the same number,
+ * and it keeps describing the stored CSR while edits are pending. */
 int  kr_matrix_info(const kr_matrix* A, int64_t* n, int64_t* nnz, int* symmetric, int* pattern_only,
                     int* nonnegative);
 /* A(i,j) = A(j,i) = v for count 1-based pairs; v = 0 deletes the entry

@@ -228,11 +228,36 @@ int kr_matrix_info(const kr_matrix* A, int64_t* n, int64_t* nnz, int* symmetric,
                    int* nonnegative) {
     return guarded([&] {
         if (!A) fail(KR_ERR_ARG, "null matrix");
+        // A = stored CSR + pending edits (kr_matrix_set_edges).  Describe the edited matrix without folding the edits
+        // in, so that asking does not change which kernels the next call runs: every pending entry creates, keeps or
+        // removes one stored entry, and only an edit that clears a stored negative value needs a rescan.
+        const CsrHost& H = A->host;
+        int64_t count = A->dev.nnz;
+        bool neg_edit = false, neg_cleared = false;
+        for (const auto& kv : A->pending) {
+            const int64_t i = kv.first.first, j = kv.first.second;
+            const int32_t* b = H.col.data() + H.row_ptr[i];
+            const int32_t* e = H.col.data() + H.row_ptr[i + 1];
+            const int32_t* q = std::lower_bound(b, e, (int32_t)j);
+            const bool stored = q != e && *q == (int32_t)j;
+            const double old = stored ? H.val[(size_t)(q - H.col.data())] : 0.0;
+            const double now = old + kv.second;              // the value flush_pending stores
+            count += (int64_t)(now != 0.0) - (int64_t)stored;
+            neg_edit = neg_edit || now < 0;
+            neg_cleared = neg_cleared || (old < 0 && !(now < 0));
+        }
+        bool nonneg = A->nonnegative && !neg_edit;
+        if (!A->nonnegative && !neg_edit && neg_cleared) {   // is any stored negative left that no edit overrides?
+            nonneg = true;
+            for (int64_t i = 0; i < H.n && nonneg; ++i)
+                for (int64_t p = H.row_ptr[i]; p < H.row_ptr[i + 1]; ++p)
+                    if (H.val[(size_t)p] < 0 && !A->pending.count({i, (int64_t)H.col[(size_t)p]})) { nonneg = false; break; }
+        }
         if (n) *n = A->dev.n;
-        if (nnz) *nnz = A->dev.nnz;
+        if (nnz) *nnz = count;
         if (symmetric) *symmetric = A->symmetric;
         if (pattern_only) *pattern_only = A->dev.pattern_only;
-        if (nonnegative) *nonnegative = A->nonnegative;
+        if (nonnegative) *nonnegative = nonneg;
     });
 }
 
