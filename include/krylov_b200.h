@@ -127,6 +127,19 @@ int  kr_trace_fun_update_edges(kr_ctx* ctx, const kr_matrix* A, int64_t nE, cons
 int  kr_trace_fun_update_edges_ex(kr_ctx* ctx, const kr_matrix* A, int64_t nE, const int64_t* E,
                                   double b_offdiag, double b_self, double tol, int64_t it, int fun,
                                   double* Xm, int64_t* iter, int* lucky);
+/* Node removal, scored for every candidate node V[h] (1-based, nV of them): Xm[h] = tr f(Ã) - tr f(A), where Ã is A
+ * with the off-diagonal entries of row and column v set to zero (a_vv kept, n unchanged).  This is
+ * trace_fun_update(A, U, B) with U = [e_v, a'], a' the off-diagonal part of row v, B = -[0 1; 1 0]
+ * (functions/trace_fun_update.m:72-124), restated without its rank-deficient block: range(U) lies in K_2(A, e_v), so
+ * K_j(A, U) = K_{j+1}(A, e_v) and step j is a single-vector Lanczos run from e_v (functions/lanczos_krylov.m:73-101,
+ * bs = 1, three-term recurrence): Gm = T_{j+1}, tGm = Gm with its (1,2) and (2,1) entries zeroed, Xm = the trace
+ * formula of :83-89 on sort(eig(tGm)), sort(eig(Gm)); stop by the lag-2 rule (:104-118) or when beta_{j+1} < 1e-8
+ * (:119-124, lucky).  iter[h] = j at the stop (at most it, 1 <= it <= 128).  A node with no off-diagonal entry scores
+ * 0 with iter 1, lucky.  Pending kr_matrix_set_edges edits count, those of v's own row included.  A must be symmetric
+ * (the reference's message otherwise).  With replicas (kr_matrix_replicate) the candidates are split contiguously
+ * across the GPUs as in kr_trace_fun_update_edges_ex; results are bit-identical run to run and across replicas. */
+int  kr_trace_fun_update_nodes(kr_ctx* ctx, const kr_matrix* A, int64_t nV, const int64_t* V, double tol, int64_t it,
+                               int fun, double* Xm, int64_t* iter, int* lucky);
 /* One round of the greedy loop, functions/krylov_miobi.m:76-124: score every candidate edge (as
  * kr_trace_fun_update_edges_ex) and select arg-min (mode 0, 'break') / arg-max (mode 1, 'make') with the reference's
  * strict first-wins comparison (:112-124).  best = 0-based index into E (-1: none), best_val = its value.

@@ -51,6 +51,7 @@ PROTOTYPES = {
                                   VP, VP, VP],
     "kr_trace_fun_update_edges_ex": [VP, VP, c_i64, VP, C.c_double, C.c_double, C.c_double, c_i64, C.c_int,
                                      VP, VP, VP],
+    "kr_trace_fun_update_nodes": [VP, VP, c_i64, VP, C.c_double, c_i64, C.c_int, VP, VP, VP],
     "kr_greedy_round": [VP, VP, c_i64, VP, C.c_double, C.c_double, C.c_double, c_i64, C.c_int, C.c_int, C.c_int,
                         c_ip, c_dp, VP, VP, VP],
     "kr_fun_update": [VP, VP, c_i64, VP, c_i64, VP, c_i64, C.c_int, C.c_double, c_i64, C.c_int,

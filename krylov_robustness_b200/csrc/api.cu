@@ -21,6 +21,7 @@
 #include "frechet.cuh"
 #include "mctrace.cuh"
 #include "nodepairs.cuh"
+#include "nodes.cuh"
 
 using namespace kr;
 

@@ -21,7 +21,8 @@ __all__ = ["slq_trace", "lanczos_krylov", "arnoldi_krylov", "trace_fun_update", 
            "fun_update", "function_multiple_entries", "fun_and_grad_krylov_exp", "fun_and_grad_krylov_fun",
            "normest", "normAm", "select_taylor_degree", "expmv", "ExpmvHandle", "mc_trace", "trace_exp",
            "edge2low_rank", "compute_centrality", "find_top_edges", "find_top_missing_edges",
-           "select_candidate", "greedy_round", "krylov_miobi", "greedy_krylov", "KrylovParams", "fun_and_grad_all_edges", "hessianfcn_exp", "hessianfcn_fun"]
+           "select_candidate", "greedy_round", "krylov_miobi", "greedy_krylov", "trace_fun_update_nodes", "greedy_krylov_nodes",
+           "KrylovParams", "fun_and_grad_all_edges", "hessianfcn_exp", "hessianfcn_fun"]
 
 
 def _mat(A, ctx=None):
@@ -179,6 +180,22 @@ def trace_fun_update_edges(A, E, b_offdiag, tol=1e-12, it=None, fun="exp", b_sel
     check(M.ctx.lib.kr_trace_fun_update_edges_ex(M.ctx.h, M.h, nE, _ptr(E), float(b_offdiag),
                                                  float(b_offdiag if b_self is None else b_self), float(tol), it,
                                                  fun_id(fun), _ptr(x), _ptr(k), _ptr(lucky)))
+    return x, k, lucky.astype(bool)
+
+
+def trace_fun_update_nodes(A, nodes, tol=1e-12, it=None, fun="exp"):
+    """Node-removal scores, all candidates in one call (kr_trace_fun_update_nodes): for every node v (1-based)
+    tr f(Ã) - tr f(A), Ã = A with the off-diagonal entries of row and column v set to zero (a_vv kept).  The
+    reference's trace_fun_update (functions/trace_fun_update.m:72-124) with U = [e_v, a'], B = -[0 1; 1 0], run as a
+    single-vector Lanczos from e_v; same lag-2 and lucky-breakdown stops.  Returns (Xm, iter, lucky) arrays."""
+    M = _mat(A)
+    it = _default_it(M, it)
+    V = np.ascontiguousarray(np.asarray(nodes).ravel(), dtype=np.int64)
+    x = np.zeros(V.size)
+    k = np.zeros(V.size, dtype=np.int64)
+    lucky = np.zeros(V.size, dtype=np.int32)
+    check(M.ctx.lib.kr_trace_fun_update_nodes(M.ctx.h, M.h, V.size, _ptr(V), float(tol), it, fun_id(fun), _ptr(x),
+                                              _ptr(k), _ptr(lucky)))
     return x, k, lucky.astype(bool)
 
 
@@ -612,6 +629,45 @@ def greedy_krylov(A, k, Q=0, centrality=None, order="mult", tol=1e-12, it=None, 
     A = A.tocsr()
     A.eliminate_zeros()
     return edges, rob_variation, A
+
+
+def greedy_krylov_nodes(A, k, Q=0, centrality=None, tol=1e-12, it=None, fun="exp"):
+    """[nodes,rob_variation,A_new]: greedy node attack, the node counterpart of greedy_krylov (functions/greedy_krylov.m).
+    Round 1 ranks the nodes by centrality (descending, stable) and keeps the top Q + k; every round scores the first Q
+    remaining nodes in one trace_fun_update_nodes call, takes the first-wins arg-min (select_candidate(..., 'break')),
+    deletes the chosen node's off-diagonal entries with one in-place set_edges call and drops it from the list.  A stays
+    on the device across the rounds.  Q = 0 takes the reference's default, the largest column sum of A; centrality =
+    None computes the 'eig' centrality on the device.  Returns nodes (1-based), the summed scores and the edited A."""
+    if not _issymmetric(A):
+        raise ValueError("GREEDY_KRYLOV:: Adjacency matrix should be symmetric")
+    A = sp.csr_matrix(A).astype(np.float64)
+    n = A.shape[0]
+    it = int(min(100, n)) if it is None else int(it)
+    if not Q:
+        Q = int(np.asarray(A.sum(axis=0)).max())
+    M = Matrix(A)
+    if centrality is None:
+        centrality = compute_centrality(M, "eig")
+    top = np.argsort(-np.asarray(centrality, dtype=np.float64).ravel(), kind="stable")[:Q + k] + 1
+    A = A.tolil()
+    nodes, rob_variation = [], 0.0
+    for _ in range(min(k, top.size)):
+        cand = top[:Q]
+        vals = trace_fun_update_nodes(M, cand, tol, it, fun)[0]
+        best, bestval = select_candidate(vals, "break")
+        chosen = int(cand[best])
+        nbrs = [j + 1 for j in A.rows[chosen - 1] if j != chosen - 1]
+        if nbrs:
+            M.set_edges(np.full(len(nbrs), chosen), nbrs, 0.0)
+            for j in nbrs:
+                A[chosen - 1, j - 1] = 0.0
+                A[j - 1, chosen - 1] = 0.0
+        top = top[top != chosen]
+        nodes.append(chosen)
+        rob_variation += bestval
+    A = A.tocsr()
+    A.eliminate_zeros()
+    return np.asarray(nodes, dtype=np.int64), rob_variation, A
 
 
 def fun_and_grad_all_edges(X, A, Omega, fun, dfun, tol=1e-8, it=None):

@@ -206,7 +206,19 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         if (nlhs > 1) { plhs[1] = mxCreateDoubleMatrix(nE, 1, mxREAL); for (i = 0; i < nE; ++i) mxGetPr(plhs[1])[i] = (double)it[i]; }
         if (nlhs > 2) { plhs[2] = mxCreateDoubleMatrix(nE, 1, mxREAL); for (i = 0; i < nE; ++i) mxGetPr(plhs[2])[i] = (double)lk[i]; }
         mxFree(E); mxFree(it); mxFree(lk);
-    } else if (!strcmp(op, "greedy_round")) {                      /* [best,val,nexact] = (A,E,b,tol,it,fun,b_self,mode,screen) */
+    } else if (!strcmp(op, "trace_fun_update_nodes")) {            /* [Xm,iter,lucky] = (A,V,tol,it,fun): node removal */
+        kr_matrix* M = matrix_of(prhs[0]);
+        mwSize nV = 0, i;
+        int64_t* V = to_i64(prhs[1], &nV);
+        int64_t* it = (int64_t*)mxMalloc((nV ? nV : 1) * sizeof(int64_t));
+        int* lk = (int*)mxMalloc((nV ? nV : 1) * sizeof(int));
+        plhs[0] = mxCreateDoubleMatrix(nV, 1, mxREAL);
+        chk(kr_trace_fun_update_nodes(ctx(), M, (int64_t)nV, V, mxGetScalar(prhs[2]), (int64_t)mxGetScalar(prhs[3]),
+                                      fun_of(prhs[4]), mxGetPr(plhs[0]), it, lk));
+        if (nlhs > 1) { plhs[1] = mxCreateDoubleMatrix(nV, 1, mxREAL); for (i = 0; i < nV; ++i) mxGetPr(plhs[1])[i] = (double)it[i]; }
+        if (nlhs > 2) { plhs[2] = mxCreateDoubleMatrix(nV, 1, mxREAL); for (i = 0; i < nV; ++i) mxGetPr(plhs[2])[i] = (double)lk[i]; }
+        mxFree(V); mxFree(it); mxFree(lk);
+    } else if (!strcmp(op, "greedy_round")) {                     /* [best,val,nexact] = (A,E,b,tol,it,fun,b_self,mode,screen) */
         /* the loop body of functions/krylov_miobi.m:76-124 in one call: candidate scores + first-wins arg-min (mode 0) /
          * arg-max (mode 1); best is the 1-based row of E (0: none).  screen = -1 reads KR_GREEDY_SCREEN. */
         kr_matrix* M = matrix_of(prhs[0]);
