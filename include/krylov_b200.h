@@ -168,6 +168,22 @@ int  kr_fun_update_fetch(kr_ctx* ctx, double* Xm, int64_t ldx, double* Um, int64
  * Environment (testing): KR_ENTRIES_LOCAL=0 dense batch only, KR_ENTRIES_CHUNK_COLS=c columns per dense chunk. */
 int  kr_function_multiple_entries(kr_ctx* ctx, const kr_matrix* A, int64_t k, const int64_t* omega,
                                   int fun, double tol, int64_t it, double* X, int64_t* iter);
+/* Objective of the all-edges callback (functions/fun_and_grad_krylov_fun.m:65 with Omega = all edges) without two
+ * large traces that cancel: dtr = tr f(Atilde) - tr f(Atilde - D), where D = Delta(X, Omega) is the symmetric sparse matrix
+ * with D(i,j) = D(j,i) = X[h] for every row (i, j) of Omega (nomega x 2 col-major, 1-based; duplicates add up, a diagonal
+ * pair gives D(i,i) = X[h]).  With A_t = Atilde - (1 - t) D, dtr = int_0^1 sum_h c_h X_h f'(A_t)(i_h, j_h) dt (c_h = 2 off
+ * the diagonal, 1 on it; f' = exp / cosh / sinh for exp / sinh / cosh) by q-point Gauss-Legendre, each node one set of
+ * entries as in kr_function_multiple_entries (same tol and it, same local / dense paths; the local path runs every
+ * (start node, quadrature node) pair in one launch per budget tier).  q is the smallest order whose error bound
+ * (q!)^4 / ((2q+1) ((2q)!)^3) n ||D||^{2q} e^{||Atilde|| + ||D||} (||D|| <= its inf-norm, ||Atilde|| by normest) is at
+ * most tol * sum_h c_h |X_h|, capped at min(qmax, 32); q_used reports it, iter the largest step count of any entry.
+ * X = 0 gives exactly 0 with q_used = 0.  Atilde must be symmetric (the reference's message otherwise); pending
+ * kr_matrix_set_edges edits are folded in first.  The entries stay on the device and are reduced in a fixed order:
+ * results are bit-identical run to run.  info (may be NULL): {columns run by local tiers 1, 2, 3, columns through the
+ * dense batch}, a column being one (start node, quadrature node) pair. */
+int  kr_trace_fun_sparse_update(kr_ctx* ctx, const kr_matrix* Atilde, int64_t nomega, const int64_t* Omega,
+                                const double* X, int fun, double tol, int64_t it, int64_t qmax, double* dtr,
+                                int64_t* q_used, int64_t* iter, int64_t* info);
 /* [f,gr] = fun_and_grad_krylov_exp(X,A,Omega,eA,tol,it,debug)   functions/fun_and_grad_krylov_exp.m:1-113
  * [f,gr] = fun_and_grad_krylov_fun(X,A,Omega,fun,dfun,dfA,...)  functions/fun_and_grad_krylov_fun.m:1-71
  * fun == dfun == KR_FUN_EXP reproduces the _exp variant (value and gradient from one fun_update). */

@@ -58,6 +58,7 @@ PROTOTYPES = {
                       c_ip, c_ip, c_intp, c_intp],
     "kr_fun_update_fetch": [VP, VP, c_i64, VP, c_i64],
     "kr_function_multiple_entries": [VP, VP, c_i64, VP, C.c_int, C.c_double, c_i64, VP, c_ip],
+    "kr_trace_fun_sparse_update": [VP, VP, c_i64, VP, VP, C.c_int, C.c_double, c_i64, c_i64, VP, VP, VP, VP],
     "kr_fun_and_grad_krylov": [VP, VP, c_i64, VP, VP, C.c_int, C.c_int, VP, C.c_double, c_i64,
                                c_dp, VP],
     "kr_frechet_hessian": [VP, VP, c_i64, VP, C.c_int, C.c_double, c_i64, VP, c_ip],

@@ -22,6 +22,7 @@
 #include "mctrace.cuh"
 #include "nodepairs.cuh"
 #include "nodes.cuh"
+#include "sparse_update.cuh"
 
 using namespace kr;
 

@@ -14,7 +14,10 @@
 // more) goes through the dense batch: results do not depend
 // on which path a column took beyond rounding (test_gpu_krylov.py::test_function_multiple_entries_local_vs_dense).
 // Needs a symmetric stored pattern (w's support is found from the rows of v's support) and no pending edge edits.
+// The direction flavour (DIR = true, kr_trace_fun_sparse_update) runs column c on A_t = A + (t_c - 1) D instead, where D
+// is given by its values aligned with the stored CSR (zero where D has no entry): one launch serves every quadrature node.
 #pragma once
+#include <type_traits>
 #include "entries.cuh"
 
 namespace kr {
@@ -42,6 +45,13 @@ struct EntriesLocalArgs {
     int nsel;
     double tol;
 };
+
+// The direction flavour's arguments (a separate type: the default flavour's parameter block stays as it was)
+struct EntriesLocalDirArgs : EntriesLocalArgs {
+    const double* tcol;              // [R] t of column c
+    const double* dval;              // [nnz] D's values in stored CSR order
+};
+template <bool DIR> using EntriesLocalArgsOf = std::conditional_t<DIR, EntriesLocalDirArgs, EntriesLocalArgs>;
 
 __device__ __forceinline__ unsigned el_hash(int g, int hshift) { return ((unsigned)g * 2654435761u) >> hshift; }
 
@@ -192,8 +202,9 @@ __device__ __forceinline__ bool warp_tridiag_fx_taylor(const double* H, int it1,
     return true;
 }
 
+template <bool DIR>
 __global__ void __launch_bounds__(JAC_THREADS)
-entries_local_kernel(CsrDevView A, EntriesLocalArgs a) {
+entries_local_kernel(CsrDevView A, EntriesLocalArgsOf<DIR> a) {
     extern __shared__ double dyn[];
     __shared__ JacobiShared sh;
     __shared__ int s_col, s_m, s_over;
@@ -227,6 +238,12 @@ entries_local_kernel(CsrDevView A, EntriesLocalArgs a) {
         for (int i = tid; i < 4 * it1; i += JAC_THREADS) ring[i] = 0.0;
         __syncthreads();
         const int h0 = (int)(a.rows[c] - 1);
+        double tm1 = 0.0;
+        const double* dv = nullptr;
+        if constexpr (DIR) {
+            tm1 = a.tcol[c] - 1.0;
+            dv = a.dval;
+        }
         if (tid == 0) {
             const unsigned s = el_hash(h0, a.hshift);
             keys[s] = h0;
@@ -306,7 +323,11 @@ entries_local_kernel(CsrDevView A, EntriesLocalArgs a) {
                 double s = 0.0;
                 for (int p = p0; p < p1; ++p) {
                     const int li = el_lookup(keys, vals, A.col[p], a.hshift, hmask);
-                    if (li >= 0 && li < lj) s += (A.val ? A.val[p] : A.uval) * vj[li];
+                    if (li >= 0 && li < lj) {
+                        double v = A.val ? A.val[p] : A.uval;
+                        if (DIR) v = fma(tm1, dv[p], v);
+                        s += v * vj[li];
+                    }
                 }
                 w[r] = s;
             }
@@ -377,9 +398,14 @@ entries_local_kernel(CsrDevView A, EntriesLocalArgs a) {
 }
 
 struct EntriesLocalResult {
-    std::vector<double> X;           // [k], valid where flag[colof[p]] == 0
+    std::vector<double> X;           // [k], valid where flag[colof[p]] == 0 (empty for the direction flavour)
     std::vector<int> steps, flag;    // [R]
+    int tier_cols[EL_NTIERS] = {};   // columns launched per budget tier
 };
+
+// Direction flavour: column c runs on A + (t[c] - 1) D (device arrays; d aligned with the stored CSR) and the entries
+// stay on the device in X (device, [k]).
+struct EntriesLocalDir { const double* t; const double* d; double* X; };
 
 inline size_t entries_local_smem(int itl, const EntriesLocalBudget& b) {
     const int it1 = itl + 1;
@@ -388,9 +414,9 @@ inline size_t entries_local_smem(int itl, const EntriesLocalBudget& b) {
 }
 
 // rows: distinct first indices (1-based); colof[p]: column of pair p; j2[p]: second index (1-based)
-inline EntriesLocalResult entries_local_run(kr_ctx* ctx, const kr_matrix* M, const std::vector<int64_t>& rows,
+inline EntriesLocalResult entries_local_run(kr_ctx* ctx, const CsrDev& M, const std::vector<int64_t>& rows,
                                             const std::vector<int>& colof, const std::vector<int64_t>& j2, int fun,
-                                            double tol, int it) {
+                                            double tol, int it, const EntriesLocalDir* dir = nullptr) {
     const int R = (int)rows.size(), k = (int)colof.size();
     EntriesLocalResult out;
     std::vector<int> pb(R + 1, 0), pl(k);
@@ -402,19 +428,19 @@ inline EntriesLocalResult entries_local_run(kr_ctx* ctx, const kr_matrix* M, con
     }
     DevBuf<int64_t> drows(ctx, R), dj2(ctx, k);
     DevBuf<int> dpb(ctx, R + 1), dpl(ctx, k), dstate(ctx, (size_t)2 * R + 1);
-    DevBuf<double> dX(ctx, k);
+    DevBuf<double> dX(ctx, dir ? 0 : k);
     drows.upload(rows.data(), R);
     dj2.upload(j2.data(), k);
     dpb.upload(pb.data(), R + 1);
     dpl.upload(pl.data(), k);
     dstate.zero();
-    dX.zero();
+    if (!dir) dX.zero();
     EntriesLocalArgs a;
     a.rows = drows.p;
     a.pair_begin = dpb.p;
     a.pair_list = dpl.p;
     a.j2 = dj2.p;
-    a.X = dX.p;
+    a.X = dir ? dir->X : dX.p;
     a.steps = dstate.p;
     a.flag = dstate.p + R;
     a.ticket = dstate.p + 2 * R;
@@ -424,9 +450,11 @@ inline EntriesLocalResult entries_local_run(kr_ctx* ctx, const kr_matrix* M, con
     a.fun = fun;
     a.tol = tol;
     static bool attr_set[64] = {};
-    if (first_use_on_device(attr_set, ctx->device))
-        KR_CUDA(cudaFuncSetAttribute(entries_local_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)entries_local_smem(EL_IT, EL_TIERS[EL_NTIERS - 1])));
+    if (first_use_on_device(attr_set, ctx->device)) {
+        const int lim = (int)entries_local_smem(EL_IT, EL_TIERS[EL_NTIERS - 1]);
+        KR_CUDA(cudaFuncSetAttribute(entries_local_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+        KR_CUDA(cudaFuncSetAttribute(entries_local_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+    }
     DevBuf<int> dsel;
     std::vector<int> sel;                                   // empty: all columns
     for (int tier = 0; tier < EL_NTIERS; ++tier) {
@@ -444,7 +472,16 @@ inline EntriesLocalResult entries_local_run(kr_ctx* ctx, const kr_matrix* M, con
         const int per_sm = std::max(1, (int)((size_t)228 * 1024 / (smem + 4096 + 1024)));      // + static + the per-CTA reserve
         const int ctas = (int)std::min<int64_t>(todo, (int64_t)ctx->num_sms * per_sm);
         KR_CUDA(cudaMemsetAsync(a.ticket, 0, sizeof(int), ctx->stream));
-        KR_LAUNCH(ctx, entries_local_kernel, ctas, JAC_THREADS, smem, M->dev.view(), a);
+        out.tier_cols[tier] = todo;
+        if (dir) {
+            EntriesLocalDirArgs da;
+            static_cast<EntriesLocalArgs&>(da) = a;
+            da.tcol = dir->t;
+            da.dval = dir->d;
+            KR_LAUNCH(ctx, entries_local_kernel<true>, ctas, JAC_THREADS, smem, M.view(), da);
+        } else {
+            KR_LAUNCH(ctx, entries_local_kernel<false>, ctas, JAC_THREADS, smem, M.view(), a);
+        }
         if (tier == EL_NTIERS - 1) break;
         // what this tier flagged goes to the next one
         std::vector<int> fl(R);
@@ -458,7 +495,7 @@ inline EntriesLocalResult entries_local_run(kr_ctx* ctx, const kr_matrix* M, con
         dsel.reset(ctx, sel.size());
         dsel.upload(sel.data(), sel.size());
     }
-    out.X = dX.to_host();
+    if (!dir) out.X = dX.to_host();
     std::vector<int> st = dstate.to_host();
     out.steps.assign(st.begin(), st.begin() + R);
     out.flag.assign(st.begin() + R, st.begin() + 2 * R);

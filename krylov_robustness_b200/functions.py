@@ -22,7 +22,7 @@ __all__ = ["slq_trace", "lanczos_krylov", "arnoldi_krylov", "trace_fun_update", 
            "normest", "normAm", "select_taylor_degree", "expmv", "ExpmvHandle", "mc_trace", "trace_exp",
            "edge2low_rank", "compute_centrality", "find_top_edges", "find_top_missing_edges",
            "select_candidate", "greedy_round", "krylov_miobi", "greedy_krylov", "trace_fun_update_nodes", "greedy_krylov_nodes",
-           "KrylovParams", "fun_and_grad_all_edges", "hessianfcn_exp", "hessianfcn_fun"]
+           "trace_fun_sparse_update", "KrylovParams", "fun_and_grad_all_edges", "hessianfcn_exp", "hessianfcn_fun"]
 
 
 def _mat(A, ctx=None):
@@ -268,6 +268,31 @@ def function_multiple_entries(A, omega, f, tol=1e-12, it=None, poles=np.inf, deb
     if itv.value == it:
         warnings.warn("FUNCTION_MULTIPLE_ENTRIES:: Reached maximum number of iterations")
     return X, itv.value
+
+
+def trace_fun_sparse_update(A, X, Omega, fun, tol=1e-12, it=None, qmax=32, return_info=False):
+    """(dtr, q, iter) with dtr = tr fun(A) - tr fun(A - D), D = Delta(X, Omega): D(i,j) = D(j,i) = X[h] for every row
+    (i, j) of Omega (1-based; duplicates add up, a diagonal pair gives D(i,i) = X[h]) - so A here is the UPDATED matrix.
+    kr_trace_fun_sparse_update: q-point Gauss-Legendre along A_t = A - (1 - t) D, each node one set of entries
+    fun'(A_t)_Omega (function_multiple_entries' Krylov spaces with its tol and it); q is chosen from the quadrature's
+    error bound against tol * sum_h c_h |X_h| and capped at min(qmax, 32); iter is the largest step count of any entry.
+    Deterministic.  return_info adds {'tier_columns': [3 counts], 'dense_columns': count}, a column being one
+    (start node, quadrature node) pair of the local path (csrc/entries_local.cuh)."""
+    M = _mat(A)
+    it = _default_it(M, it)
+    Om = np.asfortranarray(np.asarray(Omega).reshape(-1, 2).astype(np.int64))
+    X = np.ascontiguousarray(np.asarray(X, dtype=np.float64).ravel())
+    if X.size != Om.shape[0]:
+        raise ValueError("X must have one value per row of Omega")
+    dtr = C.c_double()
+    q = C.c_int64()
+    itv = C.c_int64()
+    info = (C.c_int64 * 4)()
+    check(M.ctx.lib.kr_trace_fun_sparse_update(M.ctx.h, M.h, Om.shape[0], _ptr(Om), _ptr(X), fun_id(fun), float(tol),
+                                               it, int(qmax), C.byref(dtr), C.byref(q), C.byref(itv), info))
+    if return_info:
+        return dtr.value, q.value, itv.value, {"tier_columns": list(info)[:3], "dense_columns": info[3]}
+    return dtr.value, q.value, itv.value
 
 
 def _fun_and_grad(X, A, Omega, fun, dfun, dfA, tol, it):
@@ -670,7 +695,7 @@ def greedy_krylov_nodes(A, k, Q=0, centrality=None, tol=1e-12, it=None, fun="exp
     return np.asarray(nodes, dtype=np.int64), rob_variation, A
 
 
-def fun_and_grad_all_edges(X, A, Omega, fun, dfun, tol=1e-8, it=None):
+def fun_and_grad_all_edges(X, A, Omega, fun, dfun, tol=1e-8, it=None, objective=False):
     """Objective and gradient over a LARGE edge set Omega (config C2: "gradient over all edges").
 
     Calling fun_and_grad_krylov_fun literally with Omega = all edges makes U an n x n selector and the
@@ -678,17 +703,26 @@ def fun_and_grad_all_edges(X, A, Omega, fun, dfun, tol=1e-8, it=None):
     mathematically identical sparse formulation used by the reference's own Hessian callback
     (functions/hessianfcn_fun.m:5-7) is evaluated instead:
         Atilde = A + Delta(X, Omega),   gr = -2 * dfun(Atilde)_Omega   (function_multiple_entries, one
-        single-vector Krylov space per distinct row, all advanced by one wide SpMM per step),
-        f = -(trace fun(Atilde) - trace fun(A)) is NOT computed here (use slq_trace / mc_trace on both).
-    Returns gr (len(Omega))."""
+        single-vector Krylov space per distinct row, all advanced by one wide SpMM per step).
+    With objective=True the objective f = -(trace fun(Atilde) - trace fun(A)) comes too, from
+    trace_fun_sparse_update on the same device copy of Atilde with the same tol and it: a quadrature of the entries
+    fun'(A_t)_Omega along the path from A to Atilde (deterministic, to tol; the derivative is taken from fun, dfun
+    serves the gradient only).  Returns gr (len(Omega)), or (f, gr) with objective=True."""
     A = sp.csr_matrix(A).astype(np.float64)
     n = A.shape[0]
     Om = np.atleast_2d(np.asarray(Omega)).astype(np.int64)
     X = np.asarray(X, dtype=np.float64).ravel()
     D = sp.csr_matrix((X, (Om[:, 0] - 1, Om[:, 1] - 1)), shape=(n, n))
     At = (A + D + D.T).tocsr()
-    vals, _ = function_multiple_entries(At, Om, dfun, tol, it)
-    return -2.0 * vals
+    if not objective:
+        vals, _ = function_multiple_entries(At, Om, dfun, tol, it)
+        return -2.0 * vals
+    Mt = Matrix(At)
+    vals, _ = function_multiple_entries(Mt, Om, dfun, tol, it)
+    # D + D' above puts 2 X_h on the diagonal for a pair (i, i); Delta of trace_fun_sparse_update puts X_h there
+    Xd = np.where(Om[:, 0] == Om[:, 1], 2.0 * X, X)
+    dtr = trace_fun_sparse_update(Mt, Xd, Om, fun, tol, it)[0]
+    return -dtr, -2.0 * vals
 
 
 def _hessian(X, A, Omega, fun, tol, it):

@@ -258,6 +258,19 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
                                          (int64_t)mxGetScalar(prhs[4]), mxGetPr(plhs[0]), &it));
         if (nlhs > 1) plhs[1] = scalar((double)it);
         mxFree(om);
+    } else if (!strcmp(op, "trace_fun_sparse_update")) {         /* [dtr,q,iter] = (At,Omega,X,fun,tol,it,qmax) */
+        kr_matrix* M = matrix_of(prhs[0]);
+        mwSize k = mxGetM(prhs[1]);
+        int64_t* om = to_i64(prhs[1], NULL);
+        int64_t q, it;
+        double dtr;
+        if (mxGetNumberOfElements(prhs[2]) != k) mexErrMsgTxt("trace_fun_sparse_update: X must have one value per row of Omega");
+        chk(kr_trace_fun_sparse_update(ctx(), M, (int64_t)k, om, mxGetPr(prhs[2]), fun_of(prhs[3]), mxGetScalar(prhs[4]),
+                                       (int64_t)mxGetScalar(prhs[5]), (int64_t)mxGetScalar(prhs[6]), &dtr, &q, &it, NULL));
+        plhs[0] = scalar(dtr);
+        if (nlhs > 1) plhs[1] = scalar((double)q);
+        if (nlhs > 2) plhs[2] = scalar((double)it);
+        mxFree(om);
     } else if (!strcmp(op, "fun_and_grad")) {                      /* [f,gr] = (X,A,Omega,fun,dfun,dfA,tol,it) */
         kr_matrix* M = matrix_of(prhs[1]);
         mwSize k = mxGetM(prhs[2]);
