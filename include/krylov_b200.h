@@ -196,6 +196,24 @@ int  kr_fun_and_grad_krylov(kr_ctx* ctx, const kr_matrix* A, int64_t nomega, con
  * (hessianfcn_exp.m:4-7); Hes is nomega x nomega column-major; it is capped at 64 Krylov steps. */
 int  kr_frechet_hessian(kr_ctx* ctx, const kr_matrix* Atilde, int64_t nomega, const int64_t* Omega,
                         int fun, double tol, int64_t it, double* Hes, int64_t* iter);
+/* W = Hes * Y without assembling Hes: the HessianMultiplyFcn of the all-edges callbacks (functions/hessianfcn_fun.m:1-17
+ * over functions/multiple_frechet_eval.m:1-211, Atilde = A + Delta(X,Omega) assembled by the caller).  For every row h =
+ * (i, j) of Omega (nomega x 2 col-major, 1-based), U / V are the single-vector Arnoldi bases of K_s(Atilde, e_i) /
+ * K_s(Atilde, e_j), X_h the (1,2) block of f([G, e1 e1'; 0, H']) and s the pair's stop step (lag-3 rule, as
+ * kr_frechet_hessian; it is capped at 64 steps).  Then W(h, r) = -2 <X_h, U' S_r V>_F with
+ *   form 0 (objective): S_r = sum_l Y(l, r) (e_a e_b' + e_b e_a'), (a, b) = Omega(l, :) - the Hessian of
+ *                       -(tr f(Atilde) - tr f(A)) when f is the derivative of its function (dfun of the gradient);
+ *   form 1 (reference): S_r = sum_l Y(l, r) e_a e_b' - hessianfcn_fun's Hes * Y, except that Hes mirrors row l < h
+ *                       from X_l where W uses X_h (the two agree to the Krylov tolerance).
+ * Y: nomega x p (ld ldy), W: nomega x p (ld ldw).  Y = 0 gives W = 0 exactly; iter is the largest stop step of any pair.
+ * Atilde must be symmetric (the reference's message otherwise); pending kr_matrix_set_edges edits are folded in first.
+ * On a graph whose Krylov vectors stay local (road networks) one CTA runs a pair whole on the ball around its two nodes
+ * (csrc/hessp_local.cuh, budget tiers up to 24 steps); pairs that outgrow the last tier or need more steps take the dense
+ * families of kr_frechet_hessian, in chunks.  Results are bit-identical run to run.  info (may be NULL): {pairs launched
+ * on local tiers 1, 2, 3, pairs through the dense families}.  Environment (testing): KR_ENTRIES_LOCAL=0 dense only. */
+int  kr_frechet_hessian_multiply(kr_ctx* ctx, const kr_matrix* Atilde, int64_t nomega, const int64_t* Omega,
+                                 int64_t p, const double* Y, int64_t ldy, int fun, int form, double tol, int64_t it,
+                                 double* W, int64_t ldw, int64_t* iter, int64_t* info);
 /* MATLAB normest(A,tol) as used at functions/fun_and_grad_krylov_fun.m:27 */
 int  kr_normest(kr_ctx* ctx, const kr_matrix* A, double tol, double* est, int64_t* count);
 

@@ -62,6 +62,8 @@ PROTOTYPES = {
     "kr_fun_and_grad_krylov": [VP, VP, c_i64, VP, VP, C.c_int, C.c_int, VP, C.c_double, c_i64,
                                c_dp, VP],
     "kr_frechet_hessian": [VP, VP, c_i64, VP, C.c_int, C.c_double, c_i64, VP, c_ip],
+    "kr_frechet_hessian_multiply": [VP, VP, c_i64, VP, c_i64, VP, c_i64, C.c_int, C.c_int, C.c_double, c_i64, VP,
+                                    c_i64, c_ip, VP],
     "kr_normest": [VP, VP, C.c_double, c_dp, c_ip],
     "kr_compute_centrality": [VP, VP, C.c_int, C.c_double, c_i64, VP, c_ip, c_intp],
     "kr_normAm": [VP, VP, C.c_double, c_i64, c_dp, c_ip],

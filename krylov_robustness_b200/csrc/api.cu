@@ -23,6 +23,7 @@
 #include "nodepairs.cuh"
 #include "nodes.cuh"
 #include "sparse_update.cuh"
+#include "hessp_local.cuh"
 
 using namespace kr;
 

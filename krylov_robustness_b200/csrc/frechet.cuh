@@ -155,6 +155,65 @@ __global__ void hessian_assemble_kernel(const double* const* __restrict__ VI, co
     }
 }
 
+// The stepping of multiple_frechet_eval (:86-195) for the pairs omega (m x 2 col-major, 1-based, checked by the caller):
+// two ArnoldiBatch families (one space per distinct first / second index) advanced together until every pair met the
+// lag-3 rule or it steps were taken.  xfin[p] (nfin[p] x nfin[p], ld nfin[p]) is X of pair p at its stop step.
+struct FrechetPairs {
+    std::vector<int64_t> rowsI, rowsJ;
+    std::vector<int> sa, sb;
+    std::unique_ptr<ArnoldiBatch> BI, BJ;
+    DevBuf<int> dsa, dsb, istate;               // istate: nfin[m], conv[m], nactive
+    DevBuf<double> hist, xfin;
+    int64_t iter = 0;
+    const int* nfin() const { return istate.p; }
+};
+
+inline void frechet_pairs_run(kr_ctx* ctx, const kr_matrix* M, int64_t m, const int64_t* omega, int fun, double tol,
+                              int it, FrechetPairs& F) {
+    const int it1 = it + 1;
+    F.sa.resize(m);
+    F.sb.resize(m);
+    std::map<int64_t, int> pi, pj;
+    for (int64_t p = 0; p < m; ++p) {
+        const int64_t i = omega[p], j = omega[m + p];
+        auto fi = pi.find(i);
+        if (fi == pi.end()) { pi[i] = (int)F.rowsI.size(); F.sa[p] = (int)F.rowsI.size(); F.rowsI.push_back(i); } else F.sa[p] = fi->second;
+        auto fj = pj.find(j);
+        if (fj == pj.end()) { pj[j] = (int)F.rowsJ.size(); F.sb[p] = (int)F.rowsJ.size(); F.rowsJ.push_back(j); } else F.sb[p] = fj->second;
+    }
+    F.BI.reset(new ArnoldiBatch(ctx, M->dev, F.rowsI, it));
+    F.BJ.reset(new ArnoldiBatch(ctx, M->T(), F.rowsJ, it));
+    F.dsa.reset(ctx, m);
+    F.dsb.reset(ctx, m);
+    F.istate.reset(ctx, (size_t)2 * m + 1);
+    F.dsa.upload(F.sa.data(), m);
+    F.dsb.upload(F.sb.data(), m);
+    F.hist.reset(ctx, (size_t)m * 4 * FRECHET_CAP * FRECHET_CAP);
+    F.xfin.reset(ctx, (size_t)m * FRECHET_CAP * FRECHET_CAP);
+    F.hist.zero(); F.xfin.zero(); F.istate.zero();
+    int* nfin = F.istate.p;
+    int* conv = F.istate.p + m;
+    int* nactive = F.istate.p + 2 * m;
+    int nact = (int)m;
+    KR_CUDA(cudaMemcpyAsync(nactive, &nact, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    static bool attr_set[64] = {};              // per device: the attribute lives in the device's primary context
+    if (first_use_on_device(attr_set, ctx->device))
+        KR_CUDA(cudaFuncSetAttribute(frechet_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)JAC_SMEM_LIMIT));
+    int j = 0;
+    for (j = 0; j < it; ++j) {
+        F.BI->step(j);
+        F.BJ->step(j);
+        const int jj = j + 1;
+        const size_t smem = (size_t)(5 * jj * (jj | 1)) * sizeof(double);
+        KR_LAUNCH(ctx, frechet_step_kernel, (int)m, JAC_THREADS, smem, F.BI->Hc.p, F.BJ->Hc.p, it1, jj, fun, tol, F.dsa.p,
+                  F.dsb.p, F.hist.p, F.xfin.p, nfin, conv, nactive);
+        KR_CUDA(cudaMemcpyAsync(&nact, nactive, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+        KR_CUDA(cudaStreamSynchronize(ctx->stream));
+        if (nact <= 0) { ++j; break; }
+    }
+    F.iter = std::min(j, it);
+}
+
 struct HessianResult { std::vector<double> Hes; int64_t iter = 0; };
 
 // omega: m x 2 column-major on the host (1-based)
@@ -162,54 +221,115 @@ inline HessianResult frechet_hessian_run(kr_ctx* ctx, const kr_matrix* M, int64_
                                          double tol, int it) {
     const int64_t n = M->dev.n;
     it = std::min(it, FRECHET_CAP);
-    const int it1 = it + 1;
-    std::vector<int64_t> rowsI, rowsJ;
-    std::vector<int> sa(m), sb(m);
-    std::map<int64_t, int> pi, pj;
-    for (int64_t p = 0; p < m; ++p) {
-        const int64_t i = omega[p], j = omega[m + p];
-        if (i < 1 || i > n || j < 1 || j > n) fail(KR_ERR_ARG, "Omega index out of range");
-        auto fi = pi.find(i);
-        if (fi == pi.end()) { pi[i] = (int)rowsI.size(); sa[p] = (int)rowsI.size(); rowsI.push_back(i); } else sa[p] = fi->second;
-        auto fj = pj.find(j);
-        if (fj == pj.end()) { pj[j] = (int)rowsJ.size(); sb[p] = (int)rowsJ.size(); rowsJ.push_back(j); } else sb[p] = fj->second;
-    }
-    ArnoldiBatch BI(ctx, M->dev, rowsI, it), BJ(ctx, M->T(), rowsJ, it);
-    DevBuf<int> dsa(ctx, m), dsb(ctx, m), istate(ctx, (size_t)2 * m + 1);
+    for (int64_t q = 0; q < 2 * m; ++q)
+        if (omega[q] < 1 || omega[q] > n) fail(KR_ERR_ARG, "Omega index out of range");
+    FrechetPairs F;
+    frechet_pairs_run(ctx, M, m, omega, fun, tol, it, F);
     DevBuf<int64_t> dom(ctx, 2 * m);
-    dsa.upload(sa.data(), m);
-    dsb.upload(sb.data(), m);
     dom.upload(omega, 2 * m);
-    DevBuf<double> hist(ctx, (size_t)m * 4 * FRECHET_CAP * FRECHET_CAP), xfin(ctx, (size_t)m * FRECHET_CAP * FRECHET_CAP);
-    hist.zero(); xfin.zero(); istate.zero();
-    int* nfin = istate.p;
-    int* conv = istate.p + m;
-    int* nactive = istate.p + 2 * m;
-    int nact = (int)m;
-    KR_CUDA(cudaMemcpyAsync(nactive, &nact, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-    static bool attr_set[64] = {};              // per device: the attribute lives in the device's primary context
-    if (first_use_on_device(attr_set, ctx->device))
-        KR_CUDA(cudaFuncSetAttribute(frechet_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)JAC_SMEM_LIMIT));
     HessianResult out;
-    int j = 0;
-    for (j = 0; j < it; ++j) {
-        BI.step(j);
-        BJ.step(j);
-        const int jj = j + 1;
-        const size_t smem = (size_t)(5 * jj * (jj | 1)) * sizeof(double);
-        KR_LAUNCH(ctx, frechet_step_kernel, (int)m, JAC_THREADS, smem, BI.Hc.p, BJ.Hc.p, it1, jj, fun, tol, dsa.p, dsb.p,
-                  hist.p, xfin.p, nfin, conv, nactive);
-        KR_CUDA(cudaMemcpyAsync(&nact, nactive, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-        KR_CUDA(cudaStreamSynchronize(ctx->stream));
-        if (nact <= 0) { ++j; break; }
-    }
-    out.iter = std::min(j, it);
-    DevBuf<const double*> pI = BI.block_pointers(), pJ = BJ.block_pointers();
+    out.iter = F.iter;
+    DevBuf<const double*> pI = F.BI->block_pointers(), pJ = F.BJ->block_pointers();
     DevBuf<double> dH(ctx, (size_t)m * m);
     dH.zero();
-    KR_LAUNCH(ctx, hessian_assemble_kernel, (int)m, 64, 0, pI.p, pJ.p, n, dom.p, (int)m, dsa.p, dsb.p, xfin.p, nfin, dH.p);
+    KR_LAUNCH(ctx, hessian_assemble_kernel, (int)m, 64, 0, pI.p, pJ.p, n, dom.p, (int)m, F.dsa.p, F.dsb.p, F.xfin.p,
+              F.nfin(), dH.p);
     out.Hes = dH.to_host();
     return out;
+}
+
+// ----------------------------------------------------------------------------- Hessian times vectors
+// W(h, r) = -2 <X_h, U_h' S_r V_h>_F = -2 sum_e S_r(a_e, b_e) U_h(a_e, :) X_h V_h(b_e, :)'  over the entries e of S
+// (entry list sorted by (a, b), sval[e * p + r]).  One CTA per pair; the entries go in blocks of HESSP_THREADS: thread t
+// forms g_e for entry e0 + t, then thread t sums column r = r0 + t over the block in entry order.  Every sum has a
+// fixed order: results are bit-identical run to run.
+constexpr int HESSP_THREADS = 128;
+__global__ void __launch_bounds__(HESSP_THREADS)
+hessp_contract_kernel(const double* const* __restrict__ VI, const double* const* __restrict__ VJ, int64_t n,
+                      const int* __restrict__ sa, const int* __restrict__ sb, const double* __restrict__ xfin,
+                      const int* __restrict__ nfin, const int64_t* __restrict__ ea, const int64_t* __restrict__ eb,
+                      const double* __restrict__ sval, int64_t nnzS, int p, double* __restrict__ W, int64_t ldw) {
+    __shared__ double X[FRECHET_CAP * FRECHET_CAP];
+    __shared__ double g[HESSP_THREADS];
+    const int h = blockIdx.x, tid = threadIdx.x;
+    const int sz = nfin[h];
+    for (int e = tid; e < sz * sz; e += HESSP_THREADS) X[e] = xfin[(int64_t)h * FRECHET_CAP * FRECHET_CAP + e];
+    const int ca = sa[h], cb = sb[h];
+    const int64_t ca0 = (int64_t)(ca / PW) * n * PW + (ca % PW), cb0 = (int64_t)(cb / PW) * n * PW + (cb % PW);
+    for (int r0 = 0; r0 < p; r0 += HESSP_THREADS) {
+        double acc = 0.0;
+        for (int64_t e0 = 0; e0 < nnzS; e0 += HESSP_THREADS) {
+            __syncthreads();
+            const int64_t e = e0 + tid;
+            if (e < nnzS) {
+                const int64_t offa = ca0 + ea[e] * PW, offb = cb0 + eb[e] * PW;
+                double u[FRECHET_CAP];
+                bool any = false;
+                for (int k = 0; k < sz; ++k) { u[k] = VI[k][offa]; any |= u[k] != 0.0; }
+                double s = 0.0;
+                if (any)
+                    for (int c = 0; c < sz; ++c) {
+                        const double v = VJ[c][offb];
+                        if (v == 0.0) continue;
+                        double t = 0.0;
+                        for (int k = 0; k < sz; ++k) t += u[k] * X[k + c * sz];
+                        s += t * v;
+                    }
+                g[tid] = s;
+            }
+            __syncthreads();
+            const int r = r0 + tid;
+            if (r < p) {
+                const int64_t ne = nnzS - e0 < HESSP_THREADS ? nnzS - e0 : HESSP_THREADS;
+                for (int q = 0; q < ne; ++q) acc += g[q] * sval[(e0 + q) * p + r];
+            }
+        }
+        if (r0 + tid < p) W[h + (int64_t)(r0 + tid) * ldw] = -2.0 * acc;
+    }
+}
+
+// Bytes a chunk of the dense path holds, approximately: both families' bases (n x (it + 2) per space, worst case one space
+// per pair and family) and the 4 + 1 lag-3 / final X matrices of every pair.  ArnoldiBatch's Hessenberg columns, its
+// partial-sum buffers and the padding of a panel to PW columns come on top (a few percent at n = 10^5).
+constexpr size_t HESSP_DENSE_BUDGET = (size_t)16 << 30;
+
+// The pairs sel of omega (m x 2, 1-based, checked) through the dense families, in chunks that fit HESSP_DENSE_BUDGET;
+// row h of W (m x p, ld ldw, host) gets -2 <X_h, U_h' S V_h>.  S: entries (ea, eb) (0-based, sorted) with values
+// sval[e * p + r].  Returns the largest stop step of any pair.
+inline int64_t hessp_dense_run(kr_ctx* ctx, const kr_matrix* M, int64_t m, const int64_t* omega,
+                               const std::vector<int64_t>& sel, int fun, double tol, int it,
+                               const std::vector<int64_t>& ea, const std::vector<int64_t>& eb,
+                               const std::vector<double>& sval, int p, double* W, int64_t ldw) {
+    const int64_t n = M->dev.n, nnzS = (int64_t)ea.size();
+    it = std::min(it, FRECHET_CAP);
+    const size_t per_pair = (size_t)2 * (size_t)n * (it + 2) * sizeof(double) +
+                            (size_t)5 * FRECHET_CAP * FRECHET_CAP * sizeof(double);
+    const int64_t chunk = std::max<int64_t>(1, (int64_t)(HESSP_DENSE_BUDGET / per_pair));
+    DevBuf<int64_t> dea(ctx, nnzS), deb(ctx, nnzS);
+    DevBuf<double> dsv(ctx, sval.size());
+    dea.upload(ea.data(), nnzS);
+    deb.upload(eb.data(), nnzS);
+    dsv.upload(sval.data(), sval.size());
+    int64_t iter = 0;
+    for (int64_t c0 = 0; c0 < (int64_t)sel.size(); c0 += chunk) {
+        const int64_t mc = std::min<int64_t>(chunk, (int64_t)sel.size() - c0);
+        std::vector<int64_t> om(2 * mc);
+        for (int64_t q = 0; q < mc; ++q) {
+            om[q] = omega[sel[c0 + q]];
+            om[mc + q] = omega[m + sel[c0 + q]];
+        }
+        FrechetPairs F;
+        frechet_pairs_run(ctx, M, mc, om.data(), fun, tol, it, F);
+        iter = std::max(iter, F.iter);
+        DevBuf<const double*> pI = F.BI->block_pointers(), pJ = F.BJ->block_pointers();
+        DevBuf<double> dW(ctx, (size_t)mc * p);
+        KR_LAUNCH(ctx, hessp_contract_kernel, (int)mc, HESSP_THREADS, 0, pI.p, pJ.p, n, F.dsa.p, F.dsb.p, F.xfin.p,
+                  F.nfin(), dea.p, deb.p, dsv.p, nnzS, p, dW.p, mc);
+        std::vector<double> Wc = dW.to_host();
+        for (int r = 0; r < p; ++r)
+            for (int64_t q = 0; q < mc; ++q) W[sel[c0 + q] + (int64_t)r * ldw] = Wc[q + (int64_t)r * mc];
+    }
+    return iter;
 }
 
 }  // namespace kr

@@ -22,7 +22,8 @@ __all__ = ["slq_trace", "lanczos_krylov", "arnoldi_krylov", "trace_fun_update", 
            "normest", "normAm", "select_taylor_degree", "expmv", "ExpmvHandle", "mc_trace", "trace_exp",
            "edge2low_rank", "compute_centrality", "find_top_edges", "find_top_missing_edges",
            "select_candidate", "greedy_round", "krylov_miobi", "greedy_krylov", "trace_fun_update_nodes", "greedy_krylov_nodes",
-           "trace_fun_sparse_update", "KrylovParams", "fun_and_grad_all_edges", "hessianfcn_exp", "hessianfcn_fun"]
+           "trace_fun_sparse_update", "KrylovParams", "fun_and_grad_all_edges", "hessp_all_edges", "hessianfcn_exp",
+           "hessianfcn_fun"]
 
 
 def _mat(A, ctx=None):
@@ -740,6 +741,45 @@ def _hessian(X, A, Omega, fun, tol, it):
     if itv.value == int(it):
         warnings.warn("MULTIPLE_FRECHET_EVAL:: Reached maximum number of iterations")
     return Hes
+
+
+def hessp_all_edges(X, A, Omega, f, Y, tol=1e-8, it=None, reference_form=False, return_info=False):
+    """W = Hes * Y for the all-edges callbacks without assembling Hes (fmincon's HessianMultiplyFcn, SciPy's hessp):
+    kr_frechet_hessian_multiply on Atilde = A + Delta(X, Omega) (assembled as in hessianfcn_fun.m:4-7), or on A itself
+    when A is a resident Matrix of Atilde (X is then not used).  f is the function whose Frechet derivative is taken,
+    dfun of the gradient.  The default is the Hessian of the objective -(tr fun(Atilde) - tr fun(A)), whose gradient
+    fun_and_grad_all_edges returns; reference_form=True gives hessianfcn_fun's matrix times Y, which leaves out the
+    term of the mirrored direction e_b e_a' (DESIGN.md section 2).  Y is 1-D (returns 1-D) or len(Omega) x p.
+    return_info adds (iter, {'tier_pairs': [3 counts], 'dense_pairs': count})."""
+    Om = np.asfortranarray(np.asarray(Omega).reshape(-1, 2).astype(np.int64))
+    m = Om.shape[0]
+    if isinstance(A, Matrix):
+        M = A
+    else:
+        A = sp.csr_matrix(A).astype(np.float64)
+        n = A.shape[0]
+        X = np.asarray(X, dtype=np.float64).ravel()
+        XX = sp.csr_matrix((X, (Om[:, 0] - 1, Om[:, 1] - 1)), shape=(n, n))
+        M = Matrix((A + XX + XX.T).tocsr())
+    it = _default_it(M, it)
+    Y = np.asarray(Y, dtype=np.float64)
+    vec = Y.ndim == 1
+    if Y.ndim not in (1, 2) or Y.shape[0] != m:
+        raise ValueError("Y must have one row per row of Omega")
+    Yc = np.asfortranarray(Y.reshape(m, -1))
+    p = Yc.shape[1]
+    W = np.zeros((m, p), order="F")
+    itv = C.c_int64()
+    info = (C.c_int64 * 4)()
+    check(M.ctx.lib.kr_frechet_hessian_multiply(M.ctx.h, M.h, m, _ptr(Om), p, _ptr(Yc), max(m, 1), fun_id(f),
+                                                1 if reference_form else 0, float(tol), it, _ptr(W), max(m, 1),
+                                                C.byref(itv), info))
+    if itv.value == min(it, 64):
+        warnings.warn("MULTIPLE_FRECHET_EVAL:: Reached maximum number of iterations")
+    W = W[:, 0] if vec else W
+    if return_info:
+        return W, itv.value, {"tier_pairs": list(info)[:3], "dense_pairs": info[3]}
+    return W
 
 
 def hessianfcn_exp(X, A, Omega, tol, it):

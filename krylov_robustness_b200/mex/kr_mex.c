@@ -293,7 +293,20 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         chk(kr_frechet_hessian(ctx(), M, (int64_t)k, om, fun_of(prhs[2]), mxGetScalar(prhs[3]),
                                (int64_t)mxGetScalar(prhs[4]), mxGetPr(plhs[0]), &it));
         mxFree(om);
-    } else if (!strcmp(op, "normest")) {                           /* [e,cnt] = (A,tol) */
+    } else if (!strcmp(op, "hessian_multiply")) {      /* [W,iter] = (Atilde, Omega, Y, f, tol, it, reference_form) */
+        kr_matrix* M = matrix_of(prhs[0]);
+        mwSize k = mxGetM(prhs[1]);
+        int64_t* om = to_i64(prhs[1], NULL);
+        int64_t it;
+        mwSize p = mxGetN(prhs[2]);
+        if (mxGetM(prhs[2]) != k) mexErrMsgTxt("hessian_multiply: Y must have one row per row of Omega");
+        plhs[0] = mxCreateDoubleMatrix(k, p, mxREAL);
+        chk(kr_frechet_hessian_multiply(ctx(), M, (int64_t)k, om, (int64_t)p, mxGetPr(prhs[2]), (int64_t)(k ? k : 1),
+                                        fun_of(prhs[3]), mxGetScalar(prhs[6]) != 0.0, mxGetScalar(prhs[4]),
+                                        (int64_t)mxGetScalar(prhs[5]), mxGetPr(plhs[0]), (int64_t)(k ? k : 1), &it, NULL));
+        if (nlhs > 1) plhs[1] = scalar((double)it);
+        mxFree(om);
+    } else if (!strcmp(op, "normest")) {                         /* [e,cnt] = (A,tol) */
         double e; int64_t c;
         chk(kr_normest(ctx(), matrix_of(prhs[0]), mxGetScalar(prhs[1]), &e, &c));
         plhs[0] = scalar(e);
