@@ -152,6 +152,20 @@ int  kr_trace_fun_update_nodes(kr_ctx* ctx, const kr_matrix* A, int64_t nV, cons
 int  kr_greedy_round(kr_ctx* ctx, const kr_matrix* A, int64_t nE, const int64_t* E, double b_offdiag, double b_self,
                      double tol, int64_t it, int fun, int mode, int screen, int64_t* best, double* best_val,
                      double* scores, int* exact, int64_t* info);
+/* Candidate loop of functions/krylov_miobi.m:76-99 with a value per candidate: for row h = (i, j) of E (1-based,
+ * nE x 2 col-major) U = [e_i e_j], B = d[h] * [0 1; 1 0]; a self loop i == j is the rank-one update B = d[h].
+ * Everything else as kr_trace_fun_update_edges_ex (tol, it, fun, lag-2 / lucky stops of functions/trace_fun_update.m:
+ * 104-124, pending edits, replicas: d is split with E).  d[h] = -w removes an edge of weight w, d[h] = +w adds one;
+ * d[h] == 0 is scored like any other value (Xm = 0).  With d[h] == b_offdiag for every non-self-loop row and
+ * d[h] == b_self for every self loop the outputs are bitwise those of kr_trace_fun_update_edges_ex.  Errors: null d
+ * with nE > 0, a non-finite d[h], an index out of range, it < 1, an unsupported fun. */
+int  kr_trace_fun_update_edges_w(kr_ctx* ctx, const kr_matrix* A, int64_t nE, const int64_t* E, const double* d,
+                                 double tol, int64_t it, int fun, double* Xm, int64_t* iter, int* lucky);
+/* kr_greedy_round with a value per candidate (B = d[h] * [0 1; 1 0], as kr_trace_fun_update_edges_w): same screen,
+ * same margins and safety net, same first-wins selection (functions/krylov_miobi.m:112-124) on exact values. */
+int  kr_greedy_round_w(kr_ctx* ctx, const kr_matrix* A, int64_t nE, const int64_t* E, const double* d, double tol,
+                       int64_t it, int fun, int mode, int screen, int64_t* best, double* best_val, double* scores,
+                       int* exact, int64_t* info);
 /* [Xm,iter,lucky,Um] = fun_update(A,U,B,fun,tol,it,debug)       functions/fun_update.m:1-137
  * want_basis stands in for nargout == 4 (:69,:77).  Xm is returned column-major with leading
  * dimension xm_dim; Um (n x xm_dim, or the Lanczos window) only if want_basis.  Call with

@@ -54,6 +54,8 @@ PROTOTYPES = {
     "kr_trace_fun_update_nodes": [VP, VP, c_i64, VP, C.c_double, c_i64, C.c_int, VP, VP, VP],
     "kr_greedy_round": [VP, VP, c_i64, VP, C.c_double, C.c_double, C.c_double, c_i64, C.c_int, C.c_int, C.c_int,
                         c_ip, c_dp, VP, VP, VP],
+    "kr_trace_fun_update_edges_w": [VP, VP, c_i64, VP, VP, C.c_double, c_i64, C.c_int, VP, VP, VP],
+    "kr_greedy_round_w": [VP, VP, c_i64, VP, VP, C.c_double, c_i64, C.c_int, C.c_int, C.c_int, c_ip, c_dp, VP, VP, VP],
     "kr_fun_update": [VP, VP, c_i64, VP, c_i64, VP, c_i64, C.c_int, C.c_double, c_i64, C.c_int,
                       c_ip, c_ip, c_intp, c_intp],
     "kr_fun_update_fetch": [VP, VP, c_i64, VP, c_i64],

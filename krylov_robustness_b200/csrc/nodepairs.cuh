@@ -20,6 +20,7 @@
 // relative margin of 1e-6 of the approximate leader (100x the observed error), every ill-conditioned pair and every
 // pair not converged within the shared steps is re-scored by the exact path (pairs.cuh), and the reference's
 // first-wins selection runs on exact values.  The selected edge and its value are those of the exact round.
+// The per-candidate flavour (WB = true, kr_greedy_round_w) reads B's off-diagonal value from bw[candidate].
 #pragma once
 #include "entries.cuh"
 #include "pairs.cuh"
@@ -49,9 +50,23 @@ struct NodePairArgs {
     int* status;                                      // [np] 0 running, 1 converged, 2 ill-conditioned -> exact path
 };
 
+// The per-candidate flavour's arguments (pairs.cuh: PairStateW)
+struct NodePairArgsW : NodePairArgs {
+    const double* bw;                                 // [np] off-diagonal value of B per candidate
+};
+template <bool WB> using NodePairArgsOf = std::conditional_t<WB, NodePairArgsW, NodePairArgs>;
+
+// B's off-diagonal value of candidate c (read where it is used: the scalar flavour compiles as before the flavours)
+template <bool WB>
+__device__ __forceinline__ double node_pair_b(const NodePairArgsOf<WB>& a, int c) {
+    if constexpr (WB) return a.bw[c];
+    else return a.b_off;
+}
+
 // One CTA per candidate: steps s0 .. L of the pair recurrence in node coordinates.
+template <bool WB>
 __global__ void __launch_bounds__(NP_THREADS)
-node_pair_kernel(NodePairArgs a) {
+node_pair_kernel(NodePairArgsOf<WB> a) {
     __shared__ double S[(NP_MAXL + 1) * (NP_MAXL + 1)];          // S[p][q] = q_i^p . q_j^q
     __shared__ double Hi[(NP_MAXL + 1) * NP_MAXL], Hj[(NP_MAXL + 1) * NP_MAXL];   // Hbar (r, c) at [r * NP_MAXL + c]
     __shared__ double Mm[NP_MAXNN * NP_MAXNN], Lc[NP_MAXNN * NP_MAXNN];
@@ -105,7 +120,7 @@ node_pair_kernel(NodePairArgs a) {
             const double u1q = bq ? S[0 * W + qq] : (qq == 0 ? 1.0 : 0.0), u2q = bq ? (qq == 0 ? 1.0 : 0.0) : S[qq * W + 0];
             Mm[p + q * nn] = m;
             Kk[1][p + q * lda] = k;
-            Kk[0][p + q * lda] = k + a.b_off * (u1p * u2q + u2p * u1q);
+            Kk[0][p + q * lda] = k + node_pair_b<WB>(a, c) * (u1p * u2q + u2p * u1q);
         }
         __syncthreads();
         // ---- Cholesky M = Lc Lc' (serial: nn <= 14) with the smallest pivot as the conditioning signal
@@ -220,9 +235,10 @@ inline bool node_screen_applicable(const kr_matrix* M, int64_t np, int64_t disti
     return n * dpad * 8 * (NP_MAXL + 2) <= ((int64_t)96 << 30);                      // the shared bases must fit
 }
 
-// E: np pairs (1-based, i != j).  Fills approximate scores for the candidates the node bases could settle.
+// E: np pairs (1-based, i != j).  Fills approximate scores for the candidates the node bases could settle.  bw (device,
+// [np], may be null): the off-diagonal value of B per candidate, replacing b_off.
 inline NodeScreenOut node_screen_run(kr_ctx* ctx, const kr_matrix* M, const int64_t* Ei, const int64_t* Ej, int64_t np,
-                                     double b_off, double tol, int it, int fun) {
+                                     double b_off, double tol, int it, int fun, const double* bw = nullptr) {
     NodeScreenOut out;
     const CsrDev& A = M->dev;
     const int64_t n = A.n;
@@ -261,7 +277,9 @@ inline NodeScreenOut node_screen_run(kr_ctx* ctx, const kr_matrix* M, const int6
     dcj.upload(cj.data(), (size_t)np);
     dsteps.zero(); dstatus.zero(); dX.zero(); dapprox.zero();
     std::vector<DevBuf<double>> G((size_t)(NP_MAXL + 1) * (NP_MAXL + 1));
-    NodePairArgs a;
+    NodePairArgsW aw;
+    NodePairArgs& a = aw;
+    aw.bw = bw;
     for (auto& g : a.G) g = nullptr;
     a.Hc = B.Hc.p; a.it1 = B.it1; a.dpad = dpad;
     a.ci = dci.p; a.cj = dcj.p; a.np = (int)np; a.it = it; a.fun = fun;
@@ -305,7 +323,8 @@ inline NodeScreenOut node_screen_run(kr_ctx* ctx, const kr_matrix* M, const int6
         }
         a.L = L;
         a.s0 = evaluated + 1;
-        KR_LAUNCH(ctx, node_pair_kernel, (int)np, NP_THREADS, 0, a);
+        if (bw) KR_LAUNCH(ctx, node_pair_kernel<true>, (int)np, NP_THREADS, 0, aw);
+        else KR_LAUNCH(ctx, node_pair_kernel<false>, (int)np, NP_THREADS, 0, a);
         evaluated = L;
         out.status = dstatus.to_host();
         int64_t running = 0;

@@ -19,7 +19,11 @@
 // then one small CTA per slot: QR factor from the Gram (Householder conventions of LAPACK for exactly-zero
 // columns, see DESIGN.md "rank-deficient blocks"), projected matrices Gm / tGm, two Jacobi eigen-solves, the
 // trace formula and the reference's lag-2 stopping rule.
+//
+// The per-candidate flavour (WB = true, kr_trace_fun_update_edges_w) takes B = d[cand] * [0 1; 1 0] with d a device
+// array indexed by the candidate's position in the list: a re-seeded slot reads the value of the candidate it holds.
 #pragma once
+#include <type_traits>
 #include "dense.cuh"
 #include "smalldense.cuh"
 
@@ -114,6 +118,12 @@ struct PairState {
     int* res_lucky;
 };
 constexpr int PAIR_IDLE = 0, PAIR_NEW = 1, PAIR_RUN = 2;
+
+// The per-candidate flavour's state (a separate type: the scalar flavour's parameter block stays as it was)
+struct PairStateW : PairState {
+    const double* bw;  // [candidates] off-diagonal value of B, indexed like res_Xm
+};
+template <bool WB> using PairStateOf = std::conditional_t<WB, PairStateW, PairState>;
 
 // zero the two columns of every PAIR_NEW slot in the blocks P and C.  grid = (row blocks, panels)
 __global__ void __launch_bounds__(COL_THREADS)
@@ -412,8 +422,9 @@ __device__ double pair_projected_trace(const double* Hd, const double* Hs, const
 // pass C).  G3[slot][4] = {g11, g12, g22, -}; W is the panel-major block holding the orthogonalised
 // (un-normalised) new block.  gscratch (may be null): per-slot global work space used instead of shared memory
 // when the projected matrices outgrow it (2j > ~110).
+template <bool WB>
 __global__ void __launch_bounds__(JAC_THREADS)
-pair_step_kernel(PairState st, const double* __restrict__ G3, double* __restrict__ W, int64_t n, int mode,
+pair_step_kernel(PairStateOf<WB> st, const double* __restrict__ G3, double* __restrict__ W, int64_t n, int mode,
                  double* __restrict__ gscratch, int64_t gscratch_stride) {
     extern __shared__ double dyn[];
     __shared__ JacobiShared sh;
@@ -442,7 +453,9 @@ pair_step_kernel(PairState st, const double* __restrict__ G3, double* __restrict
     }
     __syncthreads();
     double* work = gscratch ? gscratch + (int64_t)h * gscratch_stride : dyn;
-    const double Xm = pair_projected_trace<JAC_THREADS>(Hd, Hs, Hr, j, st.b_off, st.fun, work, &sh);
+    double b_off = st.b_off;
+    if constexpr (WB) b_off = st.bw[st.cand[h]];
+    const double Xm = pair_projected_trace<JAC_THREADS>(Hd, Hs, Hr, j, b_off, st.fun, work, &sh);
     if (threadIdx.x == 0) {
         bool done = false;
         double* Xs = st.Xstop + h * 2;
@@ -485,9 +498,11 @@ __global__ void pair_panel_active_kernel(const int* __restrict__ flag, int nslot
 }
 
 // Scores the candidates (i_q, j_q), q < np (1-based end points, i != j, n > 130) and writes Xm / iter / lucky
-// in candidate order.  max_slots bounds the three n x (2*slots) work blocks.
+// in candidate order.  max_slots bounds the three n x (2*slots) work blocks.  bw (device, [np], may be null): the
+// off-diagonal value of B per candidate, replacing b_off.
 inline void pairs_run(kr_ctx* ctx, const kr_matrix* M, const int64_t* Ei, const int64_t* Ej, int64_t np, int64_t max_slots,
-                      double b_off, double tol, int it, int fun, double* Xm_out, int64_t* iter_out, int* lucky_out) {
+                      double b_off, double tol, int it, int fun, double* Xm_out, int64_t* iter_out, int* lucky_out,
+                      const double* bw = nullptr) {
     if (np <= 0) return;
     const CsrDev& A = M->dev;
     const int64_t n = A.n;
@@ -508,7 +523,9 @@ inline void pairs_run(kr_ctx* ctx, const kr_matrix* M, const int64_t* Ei, const 
     DevBuf<int> res_lucky(ctx, np);
     dstate.zero();
     istate.zero();
-    PairState st;
+    PairStateW stw;
+    PairState& st = stw;
+    stw.bw = bw;
     st.nslots = ns; st.it = it; st.fun = fun; st.tol = tol; st.b_off = b_off;
     double* d = dstate.p;
     st.Tp = d; d += ns * 4;
@@ -533,9 +550,10 @@ inline void pairs_run(kr_ctx* ctx, const kr_matrix* M, const int64_t* Ei, const 
     st.res_iter = res_iter.p;
     st.res_lucky = res_lucky.p;
 
-    static bool attr_set[64] = {};
-    if (first_use_on_device(attr_set, ctx->device))
-        KR_CUDA(cudaFuncSetAttribute(pair_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)JAC_SMEM_LIMIT));
+    static bool attr_set[64] = {}, attr_set_w[64] = {};
+    if (first_use_on_device(bw ? attr_set_w : attr_set, ctx->device))
+        KR_CUDA(cudaFuncSetAttribute(bw ? (const void*)pair_step_kernel<true> : (const void*)pair_step_kernel<false>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)JAC_SMEM_LIMIT));
 
     // host mirror of the slot table
     std::vector<long long> h_cand(ns, -1);
@@ -560,7 +578,9 @@ inline void pairs_run(kr_ctx* ctx, const kr_matrix* M, const int64_t* Ei, const 
     auto launch_step = [&](double* W, int mode, int jmax) {
         int64_t stride = 0;
         const size_t smem = step_smem(jmax, &stride);
-        KR_LAUNCH(ctx, pair_step_kernel, ns, JAC_THREADS, smem, st, st.G3, W, n, mode, stride ? gscratch.p : (double*)nullptr, stride);
+        double* gs = stride ? gscratch.p : (double*)nullptr;
+        if (bw) KR_LAUNCH(ctx, pair_step_kernel<true>, ns, JAC_THREADS, smem, stw, st.G3, W, n, mode, gs, stride);
+        else KR_LAUNCH(ctx, pair_step_kernel<false>, ns, JAC_THREADS, smem, st, st.G3, W, n, mode, gs, stride);
     };
     std::vector<int> free_slots(ns);
     for (int h = 0; h < ns; ++h) free_slots[h] = ns - 1 - h;     // pop from the back: slot 0 first

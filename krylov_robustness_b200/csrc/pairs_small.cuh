@@ -11,7 +11,7 @@
 // bit-reproducible run to run).
 //
 // Per-CTA work space in global memory (L1/L2 resident): three n x 2 blocks P (previous), C (current), Y (work),
-// one double2 per row.
+// one double2 per row.  The per-candidate flavour (WB = true) reads B's off-diagonal value from bw[cand].
 #pragma once
 #include "pairs.cuh"
 
@@ -40,6 +40,12 @@ struct PairSmallArgs {
     long long* res_iter;
     int* res_lucky;
 };
+
+// The per-candidate flavour's arguments (pairs.cuh: PairStateW)
+struct PairSmallArgsW : PairSmallArgs {
+    const double* bw;                   // [np] off-diagonal value of B per candidate
+};
+template <bool WB> using PairSmallArgsOf = std::conditional_t<WB, PairSmallArgsW, PairSmallArgs>;
 
 // fixed-order CTA sum of NV per-thread values; totals land in out[0..NV) (shared), valid after the trailing barrier
 template <int NV>
@@ -181,8 +187,9 @@ __device__ __forceinline__ void ps_spmv2(const PairSmallArgs& a, const double2* 
     if (A.dl_count > 0) __syncthreads();
 }
 
+template <bool WB>
 __global__ void __launch_bounds__(PS_THREADS, 1)
-pair_small_kernel(PairSmallArgs a) {
+pair_small_kernel(PairSmallArgsOf<WB> a) {
     extern __shared__ double dyn[];
     __shared__ JacobiShared sh;
     __shared__ double wred[PS_WARPS][8];
@@ -359,7 +366,9 @@ pair_small_kernel(PairSmallArgs a) {
             }
             __syncthreads();
             double* work = 2 * jj <= PS_SMEM_NN ? dyn : gwork;
-            const double Xm = pair_projected_trace<PS_THREADS>(Hd, Hs, Hr, jj, a.b_off, a.fun, work, &sh);
+            double b_off = a.b_off;
+            if constexpr (WB) b_off = a.bw[cand];
+            const double Xm = pair_projected_trace<PS_THREADS>(Hd, Hs, Hr, jj, b_off, a.fun, work, &sh);
             if (tid == 0) {
                 bool done = false;
                 if (jj <= 2) {
@@ -404,17 +413,21 @@ inline bool use_pairs_small(const kr_ctx* ctx, const kr_matrix* M, int64_t np) {
     return np <= ctx->num_sms || n <= 8192;
 }
 
-// Same contract as pairs_run (pairs.cuh); one launch, one synchronisation.
+// Same contract as pairs_run (pairs.cuh), bw included; one launch, one synchronisation.
 inline void pairs_small_run(kr_ctx* ctx, const kr_matrix* M, const int64_t* Ei, const int64_t* Ej, int64_t np, double b_off,
-                            double tol, int it, int fun, double* Xm_out, int64_t* iter_out, int* lucky_out) {
+                            double tol, int it, int fun, double* Xm_out, int64_t* iter_out, int* lucky_out,
+                            const double* bw = nullptr) {
     if (np <= 0) return;
     const CsrDev& A = M->dev;
     const int64_t n = A.n;
-    static bool attr_set[64] = {};
-    if (first_use_on_device(attr_set, ctx->device))
-        KR_CUDA(cudaFuncSetAttribute(pair_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PS_DYN_SMEM));
+    static bool attr_set[64] = {}, attr_set_w[64] = {};
+    if (first_use_on_device(bw ? attr_set_w : attr_set, ctx->device))
+        KR_CUDA(cudaFuncSetAttribute(bw ? (const void*)pair_small_kernel<true> : (const void*)pair_small_kernel<false>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PS_DYN_SMEM));
     const int ctas = (int)std::min<int64_t>(np, (int64_t)ctx->num_sms);      // 128 registers x 512 threads: one resident CTA per SM
-    PairSmallArgs a;
+    PairSmallArgsW aw;
+    PairSmallArgs& a = aw;
+    aw.bw = bw;
     a.A = A.view();
     a.rows_cta = a.rows_warp = 0;
     for (const RowTile& t : A.tiles_host) {
@@ -447,7 +460,8 @@ inline void pairs_small_run(kr_ctx* ctx, const kr_matrix* M, const int64_t* Ei, 
     a.np = (int)np; a.it = it; a.fun = fun; a.tol = tol; a.b_off = b_off;
     a.ws = ws.p; a.hbuf = hbuf.p;
     a.res_Xm = rx.p; a.res_iter = ri.p; a.res_lucky = rl.p;
-    KR_LAUNCH(ctx, pair_small_kernel, ctas, PS_THREADS, PS_DYN_SMEM, a);
+    if (bw) KR_LAUNCH(ctx, pair_small_kernel<true>, ctas, PS_THREADS, PS_DYN_SMEM, aw);
+    else KR_LAUNCH(ctx, pair_small_kernel<false>, ctas, PS_THREADS, PS_DYN_SMEM, a);
     std::vector<long long> itv((size_t)np);
     KR_CUDA(cudaMemcpyAsync(Xm_out, rx.p, np * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     KR_CUDA(cudaMemcpyAsync(itv.data(), ri.p, np * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));

@@ -23,7 +23,7 @@ __all__ = ["slq_trace", "lanczos_krylov", "arnoldi_krylov", "trace_fun_update", 
            "edge2low_rank", "compute_centrality", "find_top_edges", "find_top_missing_edges",
            "select_candidate", "greedy_round", "krylov_miobi", "greedy_krylov", "trace_fun_update_nodes", "greedy_krylov_nodes",
            "trace_fun_sparse_update", "KrylovParams", "fun_and_grad_all_edges", "hessp_all_edges", "hessianfcn_exp",
-           "hessianfcn_fun"]
+           "hessianfcn_fun", "trace_fun_update_edges_w", "greedy_round_w", "greedy_krylov_weighted"]
 
 
 def _mat(A, ctx=None):
@@ -184,6 +184,32 @@ def trace_fun_update_edges(A, E, b_offdiag, tol=1e-12, it=None, fun="exp", b_sel
     return x, k, lucky.astype(bool)
 
 
+def _edge_values(E, d, who):
+    """B's value per row of E: a scalar or one value per candidate (finiteness is checked by the library)."""
+    d = np.asarray(d, dtype=np.float64)
+    if d.ndim and d.size != E.shape[0]:
+        raise ValueError("%s: d must be a scalar or hold one value per row of E" % who)
+    return np.ascontiguousarray(np.broadcast_to(d.ravel() if d.ndim else d, (E.shape[0],)))
+
+
+def trace_fun_update_edges_w(A, E, d, tol=1e-12, it=None, fun="exp"):
+    """Weighted candidate loop (kr_trace_fun_update_edges_w): for each row h = (i, j) of E (1-based)
+    U = [e_i e_j], B = d[h]*[0 1;1 0]; a self loop i == j is the rank-one update B = d[h].  d[h] = -A(i, j) scores the
+    removal of edge (i, j) with its weight, d[h] = +w the insertion of an edge of weight w (functions/krylov_miobi.m:76-99
+    with a value per candidate).  d may be a scalar.  Returns (Xm, iter, lucky) arrays."""
+    M = _mat(A)
+    it = _default_it(M, it)
+    E = np.asfortranarray(np.atleast_2d(np.asarray(E)).astype(np.int64))
+    nE = E.shape[0]
+    d = _edge_values(E, d, "trace_fun_update_edges_w")
+    x = np.zeros(nE)
+    k = np.zeros(nE, dtype=np.int64)
+    lucky = np.zeros(nE, dtype=np.int32)
+    check(M.ctx.lib.kr_trace_fun_update_edges_w(M.ctx.h, M.h, nE, _ptr(E), _ptr(d), float(tol), it, fun_id(fun), _ptr(x),
+                                                _ptr(k), _ptr(lucky)))
+    return x, k, lucky.astype(bool)
+
+
 def trace_fun_update_nodes(A, nodes, tol=1e-12, it=None, fun="exp"):
     """Node-removal scores, all candidates in one call (kr_trace_fun_update_nodes): for every node v (1-based)
     tr f(Ã) - tr f(A), Ã = A with the off-diagonal entries of row and column v set to zero (a_vv kept).  The
@@ -222,6 +248,27 @@ def greedy_round(A, E, b_offdiag, tol=1e-12, it=None, fun="exp", miobi="break", 
                                     float(b_offdiag if b_self is None else b_self), float(tol), it, fun_id(fun),
                                     0 if miobi == "break" else 1, int(bool(screen)), C.byref(best), C.byref(bestval),
                                     _ptr(scores), _ptr(mask), _ptr(info)))
+    return (int(best.value), float(bestval.value), scores, mask.astype(bool),
+            dict(exact=int(info[0]), screened=int(info[1]), nodes=int(info[2]), levels=int(info[3])))
+
+
+def greedy_round_w(A, E, d, tol=1e-12, it=None, fun="exp", miobi="break", screen=True):
+    """greedy_round with a value per candidate (kr_greedy_round_w): B = d[h]*[0 1;1 0] for row h of E, as
+    trace_fun_update_edges_w.  Same screen, same first-wins selection on exact values; same returns as greedy_round."""
+    if miobi not in ("break", "make"):
+        raise ValueError("KRYLOV_MIOBI:: not supported option for miobi")
+    M = _mat(A)
+    it = _default_it(M, it)
+    E = np.asfortranarray(np.atleast_2d(np.asarray(E)).astype(np.int64))
+    nE = E.shape[0]
+    d = _edge_values(E, d, "greedy_round_w")
+    scores = np.zeros(nE)
+    mask = np.zeros(nE, dtype=np.int32)
+    info = np.zeros(4, dtype=np.int64)
+    best, bestval = C.c_int64(), C.c_double()
+    check(M.ctx.lib.kr_greedy_round_w(M.ctx.h, M.h, nE, _ptr(E), _ptr(d), float(tol), it, fun_id(fun),
+                                      0 if miobi == "break" else 1, int(bool(screen)), C.byref(best), C.byref(bestval),
+                                      _ptr(scores), _ptr(mask), _ptr(info)))
     return (int(best.value), float(bestval.value), scores, mask.astype(bool),
             dict(exact=int(info[0]), screened=int(info[1]), nodes=int(info[2]), levels=int(info[3])))
 
@@ -655,6 +702,69 @@ def greedy_krylov(A, k, Q=0, centrality=None, order="mult", tol=1e-12, it=None, 
     A = A.tocsr()
     A.eliminate_zeros()
     return edges, rob_variation, A
+
+
+def greedy_krylov_weighted(A, k, Q=0, centrality=None, order="mult", tol=1e-12, it=None, fun="exp", miobi="break",
+                           weights=None, screen=False):
+    """[edges,rob_variation,A_new,applied]: greedy_krylov on a weighted graph, scoring the change each edit makes.
+    'break': the candidates are find_top_edges(A, centrality, Q + k, order) and candidate (i, j) scores B = -A(i, j)
+    [0 1; 1 0], A(i, j) read from the current (edited) A; the chosen edge is set to 0.  'make': the candidates are
+    find_top_missing_edges(A, centrality, Q + k, order), ``weights`` is a scalar or an array aligned with that list
+    (default 1), candidate h scores B = +w_h [0 1; 1 0] and the chosen pair is set to w_h.  Each round scores the first
+    Q remaining candidates in one trace_fun_update_edges_w call (greedy_round_w with ``screen``), takes the first-wins
+    extremum (select_candidate) and applies exactly the scored change with one in-place set_edges call on the resident
+    A.  Q = 0 takes the largest column sum of A, centrality = None the 'eig' centrality on the device.  On a 0/1 graph
+    with weights = None the rounds are those of greedy_krylov.  Returns the chosen edges (1-based), the summed scores,
+    the edited A and the applied changes (A_new(i, j) - A(i, j) of each chosen edge)."""
+    if not _issymmetric(A):
+        raise ValueError("GREEDY_KRYLOV:: Adjacency matrix should be symmetric")
+    if miobi not in ("break", "make"):
+        raise ValueError("KRYLOV_MIOBI:: not supported option for miobi")
+    if miobi == "break" and weights is not None:
+        raise ValueError("greedy_krylov_weighted: weights apply to 'make' only ('break' removes the stored weight)")
+    A = sp.csr_matrix(A).astype(np.float64)
+    n = A.shape[0]
+    it = int(min(100, n)) if it is None else int(it)
+    if not Q:
+        Q = int(np.asarray(A.sum(axis=0)).max())
+    if miobi == "break" and A.nnz < 2 * k:
+        raise ValueError("GREEDY_KRYLOV:: edges to be removed are more than edges in the network")
+    M = Matrix(A)
+    if centrality is None:
+        centrality = compute_centrality(M, "eig")
+    top = (find_top_missing_edges if miobi == "make" else find_top_edges)(A, centrality, Q + k, order)
+    w = None
+    if miobi == "make":
+        w = np.asarray(1.0 if weights is None else weights, dtype=np.float64)
+        if w.ndim and w.size != top.shape[0]:
+            raise ValueError("greedy_krylov_weighted: weights must be a scalar or align with the %d candidates"
+                             % top.shape[0])
+        w = np.array(np.broadcast_to(w, (top.shape[0],)))
+    A = A.tolil()
+    rob_variation, edges, applied = 0.0, np.zeros((0, 2), dtype=np.int64), []
+    chosen = None
+    for j in range(1, min(k, top.shape[0]) + 1):
+        if j > 1:
+            keep = ~np.all(top == chosen, axis=1)                                # greedy_krylov.m:84-86
+            top = top[keep]
+            w = w[keep] if w is not None else None
+        E = top[:Q]
+        d = w[:E.shape[0]] if w is not None else -A[E[:, 0] - 1, E[:, 1] - 1].toarray().ravel()
+        if screen:
+            best, bestval = greedy_round_w(M, E, d, tol, it, fun, miobi, True)[:2]
+        else:
+            best, bestval = select_candidate(trace_fun_update_edges_w(M, E, d, tol, it, fun)[0], miobi)
+        chosen = E[best].copy()
+        newval = float(d[best]) if miobi == "make" else 0.0
+        M.set_edges([chosen[0]], [chosen[1]], newval)
+        A[chosen[0] - 1, chosen[1] - 1] = newval
+        A[chosen[1] - 1, chosen[0] - 1] = newval
+        edges = np.vstack([edges, chosen[None, :]])
+        rob_variation += bestval
+        applied.append(float(d[best]))
+    A = A.tocsr()
+    A.eliminate_zeros()
+    return edges, rob_variation, A, np.asarray(applied)
 
 
 def greedy_krylov_nodes(A, k, Q=0, centrality=None, tol=1e-12, it=None, fun="exp"):

@@ -206,6 +206,19 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         if (nlhs > 1) { plhs[1] = mxCreateDoubleMatrix(nE, 1, mxREAL); for (i = 0; i < nE; ++i) mxGetPr(plhs[1])[i] = (double)it[i]; }
         if (nlhs > 2) { plhs[2] = mxCreateDoubleMatrix(nE, 1, mxREAL); for (i = 0; i < nE; ++i) mxGetPr(plhs[2])[i] = (double)lk[i]; }
         mxFree(E); mxFree(it); mxFree(lk);
+    } else if (!strcmp(op, "trace_fun_update_edges_w")) {          /* [Xm,iter,lucky] = (A,E,d,tol,it,fun): B = d(h)*[0 1;1 0] */
+        kr_matrix* M = matrix_of(prhs[0]);
+        mwSize nE = mxGetM(prhs[1]), i;
+        if (mxGetM(prhs[2]) * mxGetN(prhs[2]) != nE) mexErrMsgTxt("kr_mex: d must hold one value per row of E");
+        int64_t* E = to_i64(prhs[1], NULL);
+        int64_t* it = (int64_t*)mxMalloc((nE ? nE : 1) * sizeof(int64_t));
+        int* lk = (int*)mxMalloc((nE ? nE : 1) * sizeof(int));
+        plhs[0] = mxCreateDoubleMatrix(nE, 1, mxREAL);
+        chk(kr_trace_fun_update_edges_w(ctx(), M, (int64_t)nE, E, mxGetPr(prhs[2]), mxGetScalar(prhs[3]),
+                                        (int64_t)mxGetScalar(prhs[4]), fun_of(prhs[5]), mxGetPr(plhs[0]), it, lk));
+        if (nlhs > 1) { plhs[1] = mxCreateDoubleMatrix(nE, 1, mxREAL); for (i = 0; i < nE; ++i) mxGetPr(plhs[1])[i] = (double)it[i]; }
+        if (nlhs > 2) { plhs[2] = mxCreateDoubleMatrix(nE, 1, mxREAL); for (i = 0; i < nE; ++i) mxGetPr(plhs[2])[i] = (double)lk[i]; }
+        mxFree(E); mxFree(it); mxFree(lk);
     } else if (!strcmp(op, "trace_fun_update_nodes")) {            /* [Xm,iter,lucky] = (A,V,tol,it,fun): node removal */
         kr_matrix* M = matrix_of(prhs[0]);
         mwSize nV = 0, i;
@@ -231,6 +244,21 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         chk(kr_greedy_round(ctx(), M, (int64_t)nE, E, mxGetScalar(prhs[2]), mxGetScalar(prhs[6]), mxGetScalar(prhs[3]),
                             (int64_t)mxGetScalar(prhs[4]), fun_of(prhs[5]), (int)mxGetScalar(prhs[7]), screen, &best, &val,
                             NULL, NULL, info));
+        plhs[0] = scalar((double)(best + 1));
+        if (nlhs > 1) plhs[1] = scalar(val);
+        if (nlhs > 2) plhs[2] = scalar((double)info[0]);
+        mxFree(E);
+    } else if (!strcmp(op, "greedy_round_w")) {                   /* [best,val,nexact] = (A,E,d,tol,it,fun,mode,screen) */
+        /* greedy_round with B = d(h)*[0 1;1 0] per candidate; best is the 1-based row of E (0: none) */
+        kr_matrix* M = matrix_of(prhs[0]);
+        mwSize nE = mxGetM(prhs[1]);
+        if (mxGetM(prhs[2]) * mxGetN(prhs[2]) != nE) mexErrMsgTxt("kr_mex: d must hold one value per row of E");
+        int64_t* E = to_i64(prhs[1], NULL);
+        int64_t best = -1, info[4] = {0, 0, 0, 0};
+        double val = 0.0;
+        chk(kr_greedy_round_w(ctx(), M, (int64_t)nE, E, mxGetPr(prhs[2]), mxGetScalar(prhs[3]), (int64_t)mxGetScalar(prhs[4]),
+                              fun_of(prhs[5]), (int)mxGetScalar(prhs[6]), (int)mxGetScalar(prhs[7]), &best, &val, NULL, NULL,
+                              info));
         plhs[0] = scalar((double)(best + 1));
         if (nlhs > 1) plhs[1] = scalar(val);
         if (nlhs > 2) plhs[2] = scalar((double)info[0]);
