@@ -32,6 +32,9 @@ static void destroy_fun_update_result(kr_ctx* c);
 struct kr_dense {
     kr_ctx* ctx;
     PanelBuf buf;
+    // int8 sign panel (the panel-major layout, one byte per entry) holding the same values as buf while they are the
+    // +-1 probes of kr_dense_fill_rademacher; empty otherwise.  Every writer of buf drops it.
+    DevBuf<signed char> sign;
 };
 
 extern "C" {
@@ -315,6 +318,7 @@ int kr_dense_upload(kr_dense* d, const double* host, int64_t ld) {
     return guarded([&] {
         if (!d || !host) fail(KR_ERR_ARG, "kr_dense_upload: null argument");
         KR_CUDA(cudaSetDevice(d->ctx->device));
+        d->sign.free();
         upload_cm(d->ctx, host, ld, d->buf);
     });
 }
@@ -332,7 +336,8 @@ int kr_dense_fill_rademacher(kr_dense* d, uint64_t seed, int64_t col_offset) {
         if (!d) fail(KR_ERR_ARG, "null block");
         KR_CUDA(cudaSetDevice(d->ctx->device));
         if (d->buf.elems() == 0) return;
-        KR_LAUNCH(d->ctx, rademacher_kernel, d->ctx->num_sms * 8, 256, 0, d->buf.p(), d->buf.n, d->buf.cols,
+        if (!d->sign.p) d->sign.reset(d->ctx, (size_t)d->buf.elems());
+        KR_LAUNCH(d->ctx, rademacher_kernel, d->ctx->num_sms * 8, 256, 0, d->buf.p(), d->sign.p, d->buf.n, d->buf.cols,
                   d->buf.panels, seed, col_offset);
     });
 }
@@ -345,6 +350,7 @@ int kr_spmm_dev(kr_ctx* ctx, const kr_matrix* A, const kr_dense* X, kr_dense* Y)
         if (Y->buf.n != X->buf.n || Y->buf.cols != X->buf.cols || Y->buf.p() == X->buf.p())
             fail(KR_ERR_ARG, "kr_spmm_dev: Y must be a distinct block of the same shape as X");
         KR_CUDA(cudaSetDevice(ctx->device));
+        Y->sign.free();
         EpiPlain epi{Y->buf.p(), X->buf.p(), 1.0, 0.0};
         launch_spmm(ctx, A->dev, X->buf.p(), X->buf.panels, epi, nullptr, X->buf.cols);
     });
@@ -382,18 +388,18 @@ int kr_slq_trace_dev(kr_ctx* ctx, const kr_matrix* A, const kr_dense* Z, int64_t
         if (!ctx || !A || !Z) fail(KR_ERR_ARG, "kr_slq_trace_dev: null argument");
         if (fun < 0 || fun > 2) fail(KR_ERR_ARG, "unsupported function selector");
         KR_CUDA(cudaSetDevice(ctx->device));
-        // work on a copy: the caller's probe block stays intact for the next step
-        PanelBuf W(ctx, Z->buf.n, Z->buf.cols);
-        KR_CUDA(cudaMemcpyAsync(W.p(), Z->buf.p(), (size_t)W.elems() * sizeof(double), cudaMemcpyDeviceToDevice,
-                                ctx->stream));
-        SlqResult R = slq_run(ctx, A, W, (int)m, fun, alpha || beta);
+        // the job only reads Z: the caller's probe block stays intact for the next step
+        const bool want_ab = alpha || beta;
+        SlqResult R = Z->sign.p ? SlqJob(ctx, A, Z->buf.n, Z->buf.cols, (const signed char*)Z->sign.p, (int)m, fun, want_ab).collect()
+                                : SlqJob(ctx, A, Z->buf.n, Z->buf.cols, (const double*)Z->buf.p(), (int)m, fun, want_ab).collect();
         slq_finish(R, m, tr, vals, alpha, beta);
     });
 }
 
 }  // extern "C"
 
-// Host-buffer SLQ pipeline shared by kr_slq_trace (fp64 probes) and kr_slq_trace_sign (int8 sign probes).
+// Host-buffer SLQ pipeline shared by kr_slq_trace (fp64 probes) and kr_slq_trace_sign (int8 sign probes, laid out
+// as int8 sign panels and never expanded to fp64).
 template <class T>
 static int slq_trace_host(kr_ctx* ctx, const kr_matrix* A, int64_t k, const T* Z, int64_t ldz, int64_t m, int fun,
                           double* tr, double* vals, double* alpha, double* beta) {
@@ -418,11 +424,10 @@ static int slq_trace_host(kr_ctx* ctx, const kr_matrix* A, int64_t k, const T* Z
         if (cstart.empty()) { cstart.push_back(0); cwidth.push_back(0); }
         const int64_t nch = (int64_t)cstart.size();
         if (!ctx->copy_stream) KR_CUDA(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-        std::vector<std::unique_ptr<PanelBuf>> W(nch);
-        std::vector<std::unique_ptr<DevBuf<T>>> stage(nch);
+        std::vector<std::unique_ptr<DevBuf<T>>> W(nch), stage(nch);      // panel-major probes, column-major staging
         std::vector<cudaEvent_t> ready(nch, nullptr);
         for (int64_t c = 0; c < nch; ++c) {
-            W[c].reset(new PanelBuf(ctx, n, (int)cwidth[c]));
+            W[c].reset(new DevBuf<T>(ctx, (size_t)n * ceil_div(cwidth[c], PW) * PW));
             stage[c].reset(new DevBuf<T>(ctx, (size_t)std::max<int64_t>(n * cwidth[c], 1)));
         }
         KR_CUDA(cudaStreamSynchronize(ctx->stream));     // pool buffers may still be in use by earlier work
@@ -433,7 +438,7 @@ static int slq_trace_host(kr_ctx* ctx, const kr_matrix* A, int64_t k, const T* Z
                                           n * sizeof(T), cw, cudaMemcpyHostToDevice, ctx->copy_stream));
                 ctx->counters[3] += n * cw * (int64_t)sizeof(T);
             }
-            cm_to_panel(ctx, stage[c]->p, n, *W[c], ctx->copy_stream);
+            cm_to_panel(ctx, stage[c]->p, n, n, (int)cw, W[c]->p, ctx->copy_stream);
             KR_CUDA(cudaEventCreateWithFlags(&ready[c], cudaEventDisableTiming));
             KR_CUDA(cudaEventRecord(ready[c], ctx->copy_stream));
         };
@@ -455,7 +460,8 @@ static int slq_trace_host(kr_ctx* ctx, const kr_matrix* A, int64_t k, const T* Z
             std::unique_ptr<SlqJob> prev;
             for (int64_t c = 0; c < nch; ++c) {
                 KR_CUDA(cudaStreamWaitEvent(ctx->stream, ready[c], 0));
-                std::unique_ptr<SlqJob> job(new SlqJob(ctx, A, *W[c], (int)m, fun, alpha || beta));   // enqueue chunk c
+                std::unique_ptr<SlqJob> job(new SlqJob(ctx, A, n, (int)cwidth[c], (const T*)W[c]->p, (int)m, fun,
+                                                       alpha || beta));   // enqueue chunk c
                 job->mark();
                 if (c + 1 < nch) issue_copy(c + 1);      // overlaps with chunk c (also when the host buffer is
                                                          // pageable and the copy call blocks)

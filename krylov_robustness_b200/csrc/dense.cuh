@@ -4,6 +4,7 @@
 // All reductions are two-stage (per-CTA partials in a fixed layout, then a fixed-order sum), never
 // float atomics, so alpha/beta and every stopping decision are bit-reproducible (SURVEY.md 7.2.2).
 #pragma once
+#include <type_traits>
 #include "spmm.cuh"
 
 namespace kr {
@@ -66,12 +67,13 @@ panel_to_cm_kernel(const double* __restrict__ src, int64_t n, int cols, double* 
     }
 }
 
-// column-major int8 signs (+1 / -1, anything else is taken by its sign, 0 stays 0) -> panel-major fp64:
-// Rademacher probes carry one bit per entry, so the host -> device copy of kr_slq_trace_sign moves 1/8 of
-// the bytes of the fp64 entry point.
+// column-major int8 signs (+1 / -1, anything else is taken by its sign, 0 stays 0) -> int8 sign panel (the
+// panel-major layout with one byte per entry, padded columns 0): Rademacher probes carry one bit per entry, so
+// the host -> device copy of kr_slq_trace_sign moves 1/8 of the bytes of the fp64 entry point, and the SLQ pass
+// reads the probes as signs (slq.cuh) without an fp64 copy.
 __global__ void __launch_bounds__(256)
 cm_i8_to_panel_kernel(const signed char* __restrict__ src, int64_t ld, int64_t n, int cols,
-                      double* __restrict__ dst) {
+                      signed char* __restrict__ dst) {
     __shared__ signed char t[PW][64 + 4];
     const int q = blockIdx.y;
     const int64_t r0 = (int64_t)blockIdx.x * 64;
@@ -82,24 +84,32 @@ cm_i8_to_panel_kernel(const signed char* __restrict__ src, int64_t ld, int64_t n
         t[c][i] = (r < n && col < cols) ? src[r + (int64_t)col * ld] : (signed char)0;
     }
     __syncthreads();
-    double* d = dst + (int64_t)q * n * PW + r0 * PW;
+    signed char* d = dst + (int64_t)q * n * PW + r0 * PW;
     for (int e = threadIdx.x; e < PW * 64; e += 256) {
         int i = e / PW, c = e % PW;
         const int v = t[c][i];
-        if (r0 + i < n) d[e] = v > 0 ? 1.0 : (v < 0 ? -1.0 : 0.0);
+        if (r0 + i < n) d[e] = (signed char)(v > 0 ? 1 : (v < 0 ? -1 : 0));
     }
 }
-inline void cm_to_panel(kr_ctx* ctx, const signed char* src_dev, int64_t ld, PanelBuf& dst, cudaStream_t stream = nullptr) {
-    if (dst.n == 0 || dst.panels == 0) return;
-    dim3 grid((unsigned)ceil_div(dst.n, 64), (unsigned)dst.panels);
-    cm_i8_to_panel_kernel<<<grid, 256, 0, stream ? stream : ctx->stream>>>(src_dev, ld, dst.n, dst.cols, dst.p());
+// n x cols column-major (ld) -> panel-major block of the same element type
+inline void cm_to_panel(kr_ctx* ctx, const signed char* src_dev, int64_t ld, int64_t n, int cols, signed char* dst,
+                        cudaStream_t stream) {
+    const int panels = (cols + PW - 1) / PW;
+    if (n == 0 || panels == 0) return;
+    dim3 grid((unsigned)ceil_div(n, 64), (unsigned)panels);
+    cm_i8_to_panel_kernel<<<grid, 256, 0, stream>>>(src_dev, ld, n, cols, dst);
     check_launch(ctx, "cm_i8_to_panel_kernel");
 }
-inline void cm_to_panel(kr_ctx* ctx, const double* src_dev, int64_t ld, PanelBuf& dst, cudaStream_t stream = nullptr) {
-    if (dst.n == 0 || dst.panels == 0) return;
-    dim3 grid((unsigned)ceil_div(dst.n, 64), (unsigned)dst.panels);
-    cm_to_panel_kernel<<<grid, 256, 0, stream ? stream : ctx->stream>>>(src_dev, ld, dst.n, dst.cols, dst.p());
+inline void cm_to_panel(kr_ctx* ctx, const double* src_dev, int64_t ld, int64_t n, int cols, double* dst,
+                        cudaStream_t stream) {
+    const int panels = (cols + PW - 1) / PW;
+    if (n == 0 || panels == 0) return;
+    dim3 grid((unsigned)ceil_div(n, 64), (unsigned)panels);
+    cm_to_panel_kernel<<<grid, 256, 0, stream>>>(src_dev, ld, n, cols, dst);
     check_launch(ctx, "cm_to_panel_kernel");
+}
+inline void cm_to_panel(kr_ctx* ctx, const double* src_dev, int64_t ld, PanelBuf& dst) {
+    cm_to_panel(ctx, src_dev, ld, dst.n, dst.cols, dst.p(), ctx->stream);
 }
 inline void panel_to_cm(kr_ctx* ctx, const PanelBuf& src, double* dst_dev, int64_t ld) {
     if (src.n == 0 || src.panels == 0) return;
@@ -107,15 +117,16 @@ inline void panel_to_cm(kr_ctx* ctx, const PanelBuf& src, double* dst_dev, int64
     KR_LAUNCH(ctx, panel_to_cm_kernel, grid, 256, 0, src.p(), src.n, src.cols, dst_dev, ld);
 }
 
-// counter-based Rademacher stream: entry (i, j) = +-1 from splitmix64(seed ^ (j << 32 | i)).
+// counter-based Rademacher stream: entry (i, j) = +-1 from splitmix64(seed ^ (j << 32 | i)).  sgn (may be null):
+// the same entries as an int8 sign panel.
 __host__ __device__ inline uint64_t splitmix64(uint64_t x) {
     x += 0x9E3779B97F4A7C15ull;
     x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
     x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
     return x ^ (x >> 31);
 }
-__global__ void rademacher_kernel(double* __restrict__ dst, int64_t n, int cols, int panels,
-                                  uint64_t seed, int64_t col_offset) {
+__global__ void rademacher_kernel(double* __restrict__ dst, signed char* __restrict__ sgn, int64_t n, int cols,
+                                  int panels, uint64_t seed, int64_t col_offset) {
     const int64_t total = n * panels * PW;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total;
          e += (int64_t)gridDim.x * blockDim.x) {
@@ -128,6 +139,7 @@ __global__ void rademacher_kernel(double* __restrict__ dst, int64_t n, int cols,
             v = (h >> 63) ? -1.0 : 1.0;
         }
         dst[e] = v;
+        if (sgn) sgn[e] = (signed char)v;
     }
 }
 
@@ -143,17 +155,25 @@ __device__ __forceinline__ void col_cta_reduce(double (&v)[NV], double* smem) {
     cta_reduce_by_sub<NV>(v, smem);      // 8 warps (COL_THREADS = 256)
 }
 
+// two adjacent entries of a panel-major block, fp64 or int8 signs
+__device__ __forceinline__ double2 ld_pair(const double* p) { return *reinterpret_cast<const double2*>(p); }
+__device__ __forceinline__ double2 ld_pair(const signed char* p) {
+    const char2 s = *reinterpret_cast<const char2*>(p);
+    return make_double2((double)(signed char)s.x, (double)(signed char)s.y);
+}
+
 // partial[rb][col] = sum over the CTA's rows of X(r,col)^2.  grid = (row_blocks, panels)
+template <class XT>
 __global__ void __launch_bounds__(COL_THREADS)
-colnorm2_kernel(const double* __restrict__ X, int64_t n, double* __restrict__ partial, int total_cols) {
+colnorm2_kernel(const XT* __restrict__ X, int64_t n, double* __restrict__ partial, int total_cols) {
     __shared__ double smem[COL_WARPS * LPT * 2];
     const int q = blockIdx.y, sub = threadIdx.x % LPT;
-    const double* Xp = X + (int64_t)q * n * PW;
+    const XT* Xp = X + (int64_t)q * n * PW;
     const int64_t r0 = (int64_t)blockIdx.x * COL_ROWS_PER_CTA;
     const int64_t r1 = min(n, r0 + COL_ROWS_PER_CTA);
     double acc[2] = {0.0, 0.0};
     for (int64_t r = r0 + (threadIdx.x / LPT); r < r1; r += COL_THREADS / LPT) {
-        double2 x = *reinterpret_cast<const double2*>(Xp + r * PW + sub * 2);
+        double2 x = ld_pair(Xp + r * PW + sub * 2);
         acc[0] += x.x * x.x;
         acc[1] += x.y * x.y;
     }
@@ -166,10 +186,14 @@ colnorm2_kernel(const double* __restrict__ X, int64_t n, double* __restrict__ pa
 }
 
 // W = c0[col]*Y + c1[col]*U1 + c2[col]*U0 (W may alias U0), partial[rb][col] = sum W^2.
-// The Lanczos three-term recurrence with per-probe coefficients (SLQ path).
+// The Lanczos three-term recurrence with per-probe coefficients (SLQ path).  U1 and U0 are fp64 or int8 sign
+// panels (T1, T0 = signed char: the probes of steps 0 and 1).  T0 = void: step 0, whose U0 is zero; the term is
+// kept as c2 * 0.0 so that the rounding is that of the three-term form.  STORE = false: the last step, where only
+// beta is needed.
+template <class T1, class T0, bool STORE = true>
 __global__ void __launch_bounds__(COL_THREADS)
-combine3_norm_kernel(const double* __restrict__ Y, const double* __restrict__ U1,
-                     const double* U0, double* W, int64_t n, const double* __restrict__ coef,
+combine3_norm_kernel(const double* __restrict__ Y, const T1* __restrict__ U1,
+                     const T0* U0, double* W, int64_t n, const double* __restrict__ coef,
                      int total_cols, double* __restrict__ partial) {
     __shared__ double smem[COL_WARPS * LPT * 2];
     const int q = blockIdx.y, sub = threadIdx.x % LPT;
@@ -184,12 +208,14 @@ combine3_norm_kernel(const double* __restrict__ Y, const double* __restrict__ U1
     for (int64_t r = r0 + (threadIdx.x / LPT); r < r1; r += COL_THREADS / LPT) {
         const int64_t o = po + r * PW + sub * 2;
         double2 y = __ldcs(reinterpret_cast<const double2*>(Y + o));
-        double2 u1 = *reinterpret_cast<const double2*>(U1 + o);
-        double2 u0 = *reinterpret_cast<const double2*>(U0 + o);
+        double2 u1 = ld_pair(U1 + o);
+        double2 u0;
+        if constexpr (std::is_void<T0>::value) u0 = make_double2(0.0, 0.0);
+        else u0 = ld_pair(U0 + o);
         double2 w;
         w.x = c0x * y.x + c1x * u1.x + c2x * u0.x;
         w.y = c0y * y.y + c1y * u1.y + c2y * u0.y;
-        *reinterpret_cast<double2*>(W + o) = w;
+        if (STORE) *reinterpret_cast<double2*>(W + o) = w;
         acc[0] += w.x * w.x;
         acc[1] += w.y * w.y;
     }

@@ -18,25 +18,33 @@ struct SlqResult {
 // One SLQ job on a panel-major probe block: enqueue() launches every kernel of the m Lanczos steps and the
 // quadrature without touching the host; collect() brings the per-probe values back.  Splitting the two
 // lets a caller overlap the host->device copy of the next column chunk with this chunk's compute.
+//
+// The probes Z are only read: they are the U1 of step 0 and the U0 of step 1.  Z is an fp64 block or an int8
+// sign panel (XT = signed char: +-1 probes at 1/8 of the bytes, the same numbers); either way every value the
+// job returns is the same to the bit.  Two work blocks P, Q and Y hold the rest: step 0 writes its W into P,
+// step 1 gathers P and writes into Q, and from step 2 on W overwrites U0.  Dropped as dead work: the U0 = 0
+// term of step 0 (its coefficient is -0 * 0), and at the last step the update and the store of Y when alpha /
+// beta are not asked for (the quadrature never reads beta_{m-1}); with them, the last update only sums |w|^2.
 struct SlqJob {
     kr_ctx* ctx;
     int m, cols, tc;
     bool want_ab;
-    PanelBuf B2, Y;
+    PanelBuf P, Q, Y;
     DevBuf<double> partial, sums, scal, alpha, beta, vals;
 
-    // Z: panel-major probes (consumed: its storage is used as a work buffer).
-    SlqJob(kr_ctx* c, const kr_matrix* M, PanelBuf& Z, int m_, int fun, bool want_ab_) : ctx(c), m(m_), want_ab(want_ab_) {
+    template <class XT>
+    SlqJob(kr_ctx* c, const kr_matrix* M, int64_t zn, int zcols, const XT* Z, int m_, int fun, bool want_ab_)
+        : ctx(c), m(m_), want_ab(want_ab_) {
         if (m < 1 || m > SLQ_MAX_M) fail(KR_ERR_ARG, "slq: m must be in 1..%d", SLQ_MAX_M);
         const CsrDev& A = M->dev;
         const int64_t n = A.n;
-        if (Z.n != n) fail(KR_ERR_ARG, "The block vector b has wrong number of rows");
-        cols = Z.cols;
-        const int panels = Z.panels;
+        if (zn != n) fail(KR_ERR_ARG, "The block vector b has wrong number of rows");
+        cols = zcols;
+        const int panels = (cols + PW - 1) / PW;
         tc = panels * PW;
-        B2.reset(ctx, n, cols);
+        P.reset(ctx, n, cols);
+        if (m > 2) Q.reset(ctx, n, cols);
         Y.reset(ctx, n, cols);
-        B2.buf.zero();
         const int rb = col_row_blocks(n);
         const int nparts = std::max(rb, A.ntiles);
         partial.reset(ctx, (size_t)nparts * tc);
@@ -55,27 +63,43 @@ struct SlqJob {
         st.alpha = alpha.p;
         st.beta = beta.p;
         const int sb = (int)ceil_div(tc, 128);
-        dim3 cgrid((unsigned)rb, (unsigned)panels);
-        KR_LAUNCH(ctx, colnorm2_kernel, cgrid, COL_THREADS, 0, Z.p(), n, partial.p, tc);
+        const dim3 cgrid((unsigned)rb, (unsigned)panels);
+        KR_LAUNCH(ctx, colnorm2_kernel, cgrid, COL_THREADS, 0, Z, n, partial.p, tc);
         sum_partials(ctx, partial.p, rb, tc, sums.p);
         KR_LAUNCH(ctx, slq_init_kernel, sb, 128, 0, sums.p, tc, st, nrm2);
-        double* U1 = Z.p();
-        double* U0 = B2.p();
+        double* U1 = P.p();
+        double* U0 = Q.p();
         for (int j = 0; j < m; ++j) {
-            EpiDot epi;
-            epi.Y = Y.p();
-            epi.X = U1;
-            epi.partial = partial.p;
-            epi.total_cols = tc;
-            launch_spmm(ctx, A, U1, panels, epi, nullptr, cols);
+            const bool last = j == m - 1;
+            const bool store = !last || want_ab;       // Y is read by this step's update
+            if (j == 0) spmm_dot(A, Z, panels, store);
+            else spmm_dot(A, (const double*)U1, panels, store);
             sum_partials(ctx, partial.p, A.ntiles, tc, sums.p);
             KR_LAUNCH(ctx, slq_alpha_kernel, sb, 128, 0, sums.p, tc, st, j);
-            KR_LAUNCH(ctx, combine3_norm_kernel, cgrid, COL_THREADS, 0, Y.p(), U1, U0, U0, n, st.coef, tc, partial.p);
+            if (!store) break;
+            if (j == 0) update(cgrid, n, Z, (const void*)nullptr, P.p(), !last);
+            else if (j == 1) update(cgrid, n, (const double*)P.p(), Z, Q.p(), !last);
+            else update(cgrid, n, (const double*)U1, (const double*)U0, U0, !last);
             sum_partials(ctx, partial.p, rb, tc, sums.p);
             KR_LAUNCH(ctx, slq_beta_kernel, sb, 128, 0, sums.p, tc, st, j);
-            std::swap(U0, U1);
+            if (j >= 1) std::swap(U0, U1);             // after step 1: U1 = Q, U0 = P
         }
         KR_LAUNCH(ctx, slq_quadrature_kernel, (int)ceil_div(cols, 64), 64, 0, alpha.p, beta.p, nrm2, m, cols, tc, fun, vals.p);
+    }
+
+    // Y = A * X with the fused alpha dot; the row operand of the dot is X itself
+    template <class XT>
+    void spmm_dot(const CsrDev& A, const XT* X, int panels, bool store) {
+        if (store) launch_spmm(ctx, A, X, panels, EpiDotT<XT, true>{Y.p(), X, partial.p, tc}, nullptr, cols);
+        else launch_spmm(ctx, A, X, panels, EpiDotT<XT, false>{Y.p(), X, partial.p, tc}, nullptr, cols);
+    }
+    template <class T1, class T0>
+    void update(dim3 cgrid, int64_t n, const T1* U1, const T0* U0, double* W, bool store) {
+        if (store)
+            combine3_norm_kernel<T1, T0, true><<<cgrid, COL_THREADS, 0, ctx->stream>>>(Y.p(), U1, U0, W, n, scal.p + 3 * tc, tc, partial.p);
+        else
+            combine3_norm_kernel<T1, T0, false><<<cgrid, COL_THREADS, 0, ctx->stream>>>(Y.p(), U1, U0, W, n, scal.p + 3 * tc, tc, partial.p);
+        check_launch(ctx, "combine3_norm_kernel");
     }
 
     // non-blocking completion marker: lets a caller enqueue the next job before waiting for this one
@@ -118,9 +142,5 @@ struct SlqJob {
     }
 };
 
-inline SlqResult slq_run(kr_ctx* ctx, const kr_matrix* M, PanelBuf& Z, int m, int fun, bool want_ab) {
-    SlqJob job(ctx, M, Z, m, fun, want_ab);
-    return job.collect();
-}
 
 }  // namespace kr

@@ -76,11 +76,28 @@ __device__ __forceinline__ Vec<4> ld_x<4>(const double* p) {
         : "=d"(r.v[0]), "=d"(r.v[1]), "=d"(r.v[2]), "=d"(r.v[3]) : "l"(p));
     return r;
 }
-__device__ __forceinline__ Vec<4> ld_row(const double* p) {           // row-local operand (plain cached load)
+// int8 sign panels (dense.cuh): the 4 signs of a lane's columns are one 32-bit word
+__device__ __forceinline__ Vec<4> signs_to_vec(unsigned w) {
+    Vec<4> r;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) r.v[i] = (double)(signed char)(w >> (8 * i));
+    return r;
+}
+template <int CPL>
+__device__ __forceinline__ Vec<CPL> ld_xv(const double* p) { return ld_x<CPL>(p); }
+template <int CPL>
+__device__ __forceinline__ Vec<CPL> ld_xv(const signed char* p) {
+    static_assert(CPL == 4, "sign gathers use 4 columns per lane");
+    return signs_to_vec(__ldg(reinterpret_cast<const unsigned*>(p)));
+}
+__device__ __forceinline__ Vec<4> ld_row(const double* p) {           // row-local operand (plain cached load)           // row-local operand (plain cached load)
     Vec<4> r;
     asm volatile("ld.global.v4.f64 {%0, %1, %2, %3}, [%4];"
                  : "=d"(r.v[0]), "=d"(r.v[1]), "=d"(r.v[2]), "=d"(r.v[3]) : "l"(p));
     return r;
+}
+__device__ __forceinline__ Vec<4> ld_row(const signed char* p) {
+    return signs_to_vec(*reinterpret_cast<const unsigned*>(p));
 }
 __device__ __forceinline__ void st_row(double* p, const Vec<4>& a) {
     asm volatile("st.global.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(p), "d"(a.v[0]), "d"(a.v[1]), "d"(a.v[2]), "d"(a.v[3]) : "memory");
@@ -97,10 +114,10 @@ __device__ __forceinline__ void st_stream(double* p, const Vec<4>& a) {
 #ifndef KR_SPMM_PF
 #define KR_SPMM_PF 1
 #endif
-__device__ __forceinline__ void prefetch_x(const double* p) {
+__device__ __forceinline__ void prefetch_x(const void* p) {
     asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
 }
-__device__ __forceinline__ void prefetch_l1(const double* p) {
+__device__ __forceinline__ void prefetch_l1(const void* p) {
     asm volatile("prefetch.global.L1 [%0];" ::"l"(p));
 }
 __device__ __forceinline__ int ld_stream(const int* p) { return __ldcs(p); }
@@ -170,10 +187,13 @@ struct EpiPlain {
 };
 
 // Y = A*X and partial[tile][col] = sum_rows X(r,col) * Y(r,col)      (Lanczos alpha, SLQ path)
-struct EpiDot {
+// XT: element type of X (double, or signed char for an int8 sign panel of +-1 probes);
+// STORE = false: the last Lanczos step, whose Y no update reads (only the dot is kept).
+template <class XT, bool STORE>
+struct EpiDotT {
     static constexpr int CPL = 4;
     double* __restrict__ Y;
-    const double* __restrict__ X;
+    const XT* __restrict__ X;
     double* __restrict__ partial;  // [ntiles][panels*PW]
     int total_cols;                // panels * PW
     double acc[CPL];
@@ -191,7 +211,7 @@ struct EpiDot {
         xr = ld_row(X + (int64_t)r * PW + sub * CPL);      // (a non-volatile load here: no gain, profiles/r02aj_*)
 #pragma unroll
         for (int i = 0; i < CPL; ++i) acc[i] += xr.v[i] * y.v[i];
-        st_stream(Y + (int64_t)r * PW + sub * CPL, y);
+        if (STORE) st_stream(Y + (int64_t)r * PW + sub * CPL, y);
     }
     __device__ __forceinline__ void finish(int tile, int panel, double* smem) {
         cta_reduce_by_sub<CPL, SPMM_WARPS, PW / CPL>(acc, smem);
@@ -202,6 +222,8 @@ struct EpiDot {
         }
     }
 };
+
+using EpiDot = EpiDotT<double, true>;
 
 // Candidate pairs (columns 2c, 2c+1): Y = A*C and raw Gram blocks P'Y, C'Y (2x2 each)
 // partial[tile][cand][8] = {P'Y (row-major 2x2), C'Y (row-major 2x2)}
@@ -442,11 +464,63 @@ __device__ __forceinline__ Vec<CPL> gather_accumulate(int p_first, int p_end, in
     return acc0;
 }
 
+// Sign flavour of the gathers (XT = signed char: an int8 panel of +-1 probes, step 0 of the SLQ pass): one 32-bit
+// load of 4 signs per lane and nonzero, a 16 B row-tile instead of 128 B.  Pattern-only A sums the signs in integers
+// (IDP4A), which is exact, so the result equals the fp64 path's sum of +-1.0 in any order.  Valued A turns the signs
+// into +-1.0 and runs the fp64 path's fma chain in its order, zero-filled partial round included: bit-identical.
+template <bool HAS_VAL, int U, bool PRED>
+__device__ __forceinline__ void sign_gather_block(int p, int p_end, int stride, const int* __restrict__ scol,
+                                                  const double* __restrict__ sval, const signed char* __restrict__ xs,
+                                                  Vec<4>& accd, int (&acci)[4]) {
+    unsigned w[U];
+    double v[U];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        const int q = p + u * stride;
+        if (PRED) {
+            w[u] = 0u;
+            v[u] = 1.0;
+        }
+        if (!PRED || q < p_end) {
+            w[u] = __ldg(reinterpret_cast<const unsigned*>(xs + (int64_t)scol[q] * PW));
+            if (HAS_VAL) v[u] = sval[q];
+        }
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        if (HAS_VAL) {
+            const Vec<4> x = signs_to_vec(w[u]);
+#pragma unroll
+            for (int i = 0; i < 4; ++i) accd.v[i] = fma(v[u], x.v[i], accd.v[i]);
+        } else {
+#pragma unroll
+            for (int i = 0; i < 4; ++i) acci[i] = __dp4a((int)w[u], 1 << (8 * i), acci[i]);
+        }
+    }
+}
+template <bool HAS_VAL, int U, int CPL>
+__device__ __forceinline__ Vec<CPL> gather_accumulate(int p_first, int p_end, int stride, const int* __restrict__ scol,
+                                                      const double* __restrict__ sval, const signed char* __restrict__ xs,
+                                                      const signed char*, int) {
+    static_assert(CPL == 4, "sign gathers use 4 columns per lane");
+    Vec<4> accd = vzero<4>();
+    int acci[4] = {0, 0, 0, 0};
+    int p = p_first;
+    for (; p + (U - 1) * stride < p_end; p += U * stride)
+        sign_gather_block<HAS_VAL, U, false>(p, p_end, stride, scol, sval, xs, accd, acci);
+    if (p < p_end) sign_gather_block<HAS_VAL, U, true>(p, p_end, stride, scol, sval, xs, accd, acci);
+    if (!HAS_VAL) {
+#pragma unroll
+        for (int i = 0; i < 4; ++i) accd.v[i] = (double)acci[i];
+    }
+    return accd;
+}
+
 // Multi-row tile: indices are already staged in shared memory; every row gets L lanes.
-template <int L, bool HAS_VAL, int U, bool DELTA, class Epi>
+template <int L, bool HAS_VAL, int U, bool DELTA, class Epi, class XT>
 __device__ __forceinline__ void spmm_tile(const RowTile t, const int* __restrict__ srp, const int* __restrict__ srid,
                                           const int* __restrict__ scol, const double* __restrict__ sval,
-                                          const double* __restrict__ Xp, double uval, Epi& epi, const CsrDevView& A,
+                                          const XT* __restrict__ Xp, double uval, Epi& epi, const CsrDevView& A,
                                           int e0, int e1) {
     constexpr int CPL = Epi::CPL;
     constexpr int LP = PW / CPL;        // lanes per row-tile
@@ -456,7 +530,7 @@ __device__ __forceinline__ void spmm_tile(const RowTile t, const int* __restrict
     const int sub = lane % LP;
     const int slot = (lane % L) / LP;
     const int rlocal = lane / L;
-    const double* xs = Xp + sub * CPL;
+    const XT* xs = Xp + sub * CPL;
     for (int base = warp * RPW; base < t.count; base += SPMM_WARPS * RPW) {
         const int rr = base + rlocal;
         const bool valid = rr < t.count;
@@ -494,7 +568,7 @@ __device__ __forceinline__ void spmm_tile(const RowTile t, const int* __restrict
         if (DELTA && e1 > e0 && emit) {   // pending edge edits of this tile (kr_matrix_set_edges): y_row += delta * x_col
             for (int e = e0; e < e1; ++e)
                 if (A.dl_rowlocal[e] == rr) {
-                    const Vec<CPL> x = ld_x<CPL>(xs + (int64_t)A.dl_col[e] * PW);
+                    const Vec<CPL> x = ld_xv<CPL>(xs + (int64_t)A.dl_col[e] * PW);
                     const double d = A.dl_val[e];
 #pragma unroll
                     for (int i = 0; i < CPL; ++i) acc.v[i] = fma(d, x.v[i], acc.v[i]);
@@ -507,8 +581,8 @@ __device__ __forceinline__ void spmm_tile(const RowTile t, const int* __restrict
 
 // One work item = (tile, panel): the CTA stages the tile's indices, serves its rows for this panel and writes the
 // epilogue's per-CTA partials.
-template <class Epi, bool HAS_VAL, int U, bool DELTA>
-__device__ __forceinline__ void spmm_item(const CsrDevView& A, const double* __restrict__ X, const Epi& epi_proto,
+template <class Epi, bool HAS_VAL, int U, bool DELTA, class XT>
+__device__ __forceinline__ void spmm_item(const CsrDevView& A, const XT* __restrict__ X, const Epi& epi_proto,
                                           int64_t panel_stride, int tile, int panel, double* red, unsigned char* dyn_smem) {
     constexpr int CPL = Epi::CPL;
     constexpr int LP = PW / CPL;
@@ -527,7 +601,7 @@ __device__ __forceinline__ void spmm_item(const CsrDevView& A, const double* __r
     const int e1 = DELTA && A.dl_tile_begin ? A.dl_tile_begin[tile + 1] : 0;
     Epi epi = epi_proto;
     epi.init(panel, panel_stride);
-    const double* Xp = X + (int64_t)panel * panel_stride;
+    const XT* Xp = X + (int64_t)panel * panel_stride;
     if (!long_row) {
         // stage the tile's row pointers, row numbers and column indices (coalesced streams)
         for (int i = threadIdx.x; i <= t.count; i += SPMM_THREADS) srp[i] = __ldg(A.row_ptr + t.start + i) - pb;
@@ -568,7 +642,7 @@ __device__ __forceinline__ void spmm_item(const CsrDevView& A, const double* __r
         for (int i = 0; i < CPL; ++i) acc.v[i] = HAS_VAL ? v[i] : v[i] * A.uval;
         if (DELTA && e1 > e0 && emit) {
             for (int e = e0; e < e1; ++e) {      // a long-row tile holds one row: every entry is its
-                const Vec<CPL> x = ld_x<CPL>(Xp + sub * CPL + (int64_t)A.dl_col[e] * PW);
+                const Vec<CPL> x = ld_xv<CPL>(Xp + sub * CPL + (int64_t)A.dl_col[e] * PW);
                 const double d = A.dl_val[e];
 #pragma unroll
                 for (int i = 0; i < CPL; ++i) acc.v[i] = fma(d, x.v[i], acc.v[i]);
@@ -582,16 +656,16 @@ __device__ __forceinline__ void spmm_item(const CsrDevView& A, const double* __r
 }
 
 // grid = (ntiles, panels); X panel q at X + q*n*PW.  `done` (may be null): skip everything if set.
-template <class Epi, bool HAS_VAL, int U, bool DELTA>
+template <class Epi, bool HAS_VAL, int U, bool DELTA, class XT>
 __global__ void __launch_bounds__(SPMM_THREADS, SPMM_MIN_CTAS)
-spmm_kernel(CsrDevView A, const double* __restrict__ X, Epi epi_proto, int64_t panel_stride,
+spmm_kernel(CsrDevView A, const XT* __restrict__ X, Epi epi_proto, int64_t panel_stride,
             const int* __restrict__ done, const int* __restrict__ panel_active) {
     if (done && *done) return;
     const int panel = blockIdx.y;
     if (panel_active && !panel_active[panel]) return;   // every column of this panel has converged
     __shared__ double red[SPMM_WARPS * LPT * 8];
     extern __shared__ __align__(16) unsigned char dyn_smem[];
-    spmm_item<Epi, HAS_VAL, U, DELTA>(A, X, epi_proto, panel_stride, (int)blockIdx.x, panel, red, dyn_smem);
+    spmm_item<Epi, HAS_VAL, U, DELTA, XT>(A, X, epi_proto, panel_stride, (int)blockIdx.x, panel, red, dyn_smem);
 }
 
 // A persistent flavour (SMs x 4 CTAs walking the (panel, tile) items in order, no CTA launch / drain per item) was
@@ -606,24 +680,24 @@ inline bool first_use_on_device(bool (&flags)[64], int device) {
     return true;
 }
 
-template <class Epi, int U>
-inline void launch_spmm_impl(kr_ctx* ctx, const CsrDev& A, const double* X, int panels, const Epi& epi,
+template <class Epi, int U, class XT>
+inline void launch_spmm_impl(kr_ctx* ctx, const CsrDev& A, const XT* X, int panels, const Epi& epi,
                              const int* done, const int* panel_active) {
     static bool attr_set[64] = {};              // one table per Epi instantiation
     if (first_use_on_device(attr_set, ctx->device)) {
-        KR_CUDA(cudaFuncSetAttribute(spmm_kernel<Epi, false, U, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPMM_SMEM_PATTERN));
-        KR_CUDA(cudaFuncSetAttribute(spmm_kernel<Epi, true, U, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPMM_SMEM_VALUED));
-        KR_CUDA(cudaFuncSetAttribute(spmm_kernel<Epi, false, U, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPMM_SMEM_PATTERN));
-        KR_CUDA(cudaFuncSetAttribute(spmm_kernel<Epi, true, U, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPMM_SMEM_VALUED));
+        KR_CUDA(cudaFuncSetAttribute(spmm_kernel<Epi, false, U, false, XT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPMM_SMEM_PATTERN));
+        KR_CUDA(cudaFuncSetAttribute(spmm_kernel<Epi, true, U, false, XT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPMM_SMEM_VALUED));
+        KR_CUDA(cudaFuncSetAttribute(spmm_kernel<Epi, false, U, true, XT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPMM_SMEM_PATTERN));
+        KR_CUDA(cudaFuncSetAttribute(spmm_kernel<Epi, true, U, true, XT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPMM_SMEM_VALUED));
     }
     const int64_t ps = (int64_t)A.n * PW;
     const dim3 grid((unsigned)A.ntiles, (unsigned)panels);
     if (A.dl_count > 0) {
-        if (A.pattern_only) spmm_kernel<Epi, false, U, true><<<grid, SPMM_THREADS, SPMM_SMEM_PATTERN, ctx->stream>>>(A.view(), X, epi, ps, done, panel_active);
-        else spmm_kernel<Epi, true, U, true><<<grid, SPMM_THREADS, SPMM_SMEM_VALUED, ctx->stream>>>(A.view(), X, epi, ps, done, panel_active);
+        if (A.pattern_only) spmm_kernel<Epi, false, U, true, XT><<<grid, SPMM_THREADS, SPMM_SMEM_PATTERN, ctx->stream>>>(A.view(), X, epi, ps, done, panel_active);
+        else spmm_kernel<Epi, true, U, true, XT><<<grid, SPMM_THREADS, SPMM_SMEM_VALUED, ctx->stream>>>(A.view(), X, epi, ps, done, panel_active);
     } else {
-        if (A.pattern_only) spmm_kernel<Epi, false, U, false><<<grid, SPMM_THREADS, SPMM_SMEM_PATTERN, ctx->stream>>>(A.view(), X, epi, ps, done, panel_active);
-        else spmm_kernel<Epi, true, U, false><<<grid, SPMM_THREADS, SPMM_SMEM_VALUED, ctx->stream>>>(A.view(), X, epi, ps, done, panel_active);
+        if (A.pattern_only) spmm_kernel<Epi, false, U, false, XT><<<grid, SPMM_THREADS, SPMM_SMEM_PATTERN, ctx->stream>>>(A.view(), X, epi, ps, done, panel_active);
+        else spmm_kernel<Epi, true, U, false, XT><<<grid, SPMM_THREADS, SPMM_SMEM_VALUED, ctx->stream>>>(A.view(), X, epi, ps, done, panel_active);
     }
 }
 
@@ -636,8 +710,8 @@ inline void launch_spmm_impl(kr_ctx* ctx, const CsrDev& A, const double* X, int 
 #endif
 
 // Host-side launcher.  Epilogues carry panel-0 pointers; init() advances them to the CTA's panel.
-template <class Epi>
-inline void launch_spmm(kr_ctx* ctx, const CsrDev& A, const double* X, int panels, const Epi& epi,
+template <class Epi, class XT>
+inline void launch_spmm(kr_ctx* ctx, const CsrDev& A, const XT* X, int panels, const Epi& epi,
                         const int* done = nullptr, int logical_cols = -1, const int* panel_active = nullptr) {
     if (A.ntiles == 0 || panels == 0) return;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
@@ -645,7 +719,7 @@ inline void launch_spmm(kr_ctx* ctx, const CsrDev& A, const double* X, int panel
         ctx->timing_events(&e0, &e1);
         KR_CUDA(cudaEventRecord(e0, ctx->stream));
     }
-    launch_spmm_impl<Epi, Epi::CPL == 4 ? KR_SPMM_U4 : KR_SPMM_U2>(ctx, A, X, panels, epi, done, panel_active);
+    launch_spmm_impl<Epi, Epi::CPL == 4 ? KR_SPMM_U4 : KR_SPMM_U2, XT>(ctx, A, X, panels, epi, done, panel_active);
     check_launch(ctx, "spmm_kernel");
     if (ctx->timing) {
         KR_CUDA(cudaEventRecord(e1, ctx->stream));
